@@ -3,7 +3,7 @@
 configs[1]: 1985-2020 x June/July/August/September inits x Pan-Arctic/Beaufort/Chukchi = 432 forecasts from
 144 SIC (57x57) + 36 SST (26x90) network builds, synthetic NSIDC-shaped monthly fields 1979-2020).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W]              # this repo's CUDA path
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--dump-outputs DIR]   # this repo's CUDA path
     python bench.py --impl reference [--steps K] [--warmup W]        # reference algorithm on the host cores
 
 One step = one pass of the whole hot path (detrend -> correlation/tau -> domain growth/merge -> node series/links
@@ -440,6 +440,38 @@ def hyper_grid_slice(torch, sw, fp64_peak):
                                                f"{rec.nbytes} result bytes"}
 
 
+RECORD_FIELDS = ("fmean", "fvar", "sigma_f", "nlml", "n_pred", "info")
+OUT_KEYS = ("_fmean", "_fvar", "_fmean_rt", "_raw_fmean", "_raw_fvar", "_raw_fmean_rt")
+
+
+def dump_outputs(dirname, sw, out, prefix=""):
+    """What one step returns to a caller of RetrospectiveSweep.run / run_many, as float64 .npy files in `dirname`:
+    `<config>.<region><key>.npy` [members, years] (the assembled forecast dict of every member) and
+    `records.<field>.npy` [problems] (the GP records `sw.raw`, in the plan's problem order).
+    A problem with no forecast (record info != 0: info = -1 where the reference's forecast() raises) comes back as NaN;
+    its entries are written as 0 and marked by `<config>.<region>_no_forecast.npy` (1.0) and `records.info.npy`, so
+    that two runs compare element by element.  Any other non-finite value is written as it is."""
+    os.makedirs(dirname, exist_ok=True)
+    failed = sw.raw["info"] != 0
+    flag = np.zeros(len(sw.raw), dtype=sw.raw.dtype)
+    flag["fmean"] = failed
+    flags = sw.plan.assemble(flag)           # same layout as `out`: 1.0 in <region>_raw_fmean where a problem failed
+    members, mflags = (out, flags) if isinstance(out, list) else ([out], [flags])
+    arrays = {}
+    for cfg in sw.cfgs:
+        for reg in cfg.regions:
+            no = np.stack([f[cfg.name][reg + "_raw_fmean"] for f in mflags]) != 0.0
+            arrays[f"{cfg.name}.{reg}_no_forecast"] = no.astype(np.float64)
+            for key in OUT_KEYS:
+                a = np.stack([np.asarray(m[cfg.name][reg + key], dtype=np.float64) for m in members])
+                arrays[f"{cfg.name}.{reg}{key}"] = np.where(no, 0.0, a)
+    for f in RECORD_FIELDS:
+        a = sw.raw[f].astype(np.float64)
+        arrays["records." + f] = a if f in ("n_pred", "info") else np.where(failed, 0.0, a)
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, prefix + name + ".npy"), a)
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -536,6 +568,8 @@ def run_ours(args):
     like_ref = int((sw.raw["info"] == -1).sum())
     other_bad = int(((sw.raw["info"] != 0) & (sw.raw["info"] != -1)).sum())
     sw.check_status(sw.raw)
+    if args.dump_outputs:                    # `out` / sw.raw: the last timed step's results
+        dump_outputs(args.dump_outputs, sw, out, prefix=f"rank{rank}." if world > 1 else "")
 
     # ---------------- strong scaling of the same step: this rank's members split over ALL ranks by (member, init, year)
     #                  task, records all-gathered as tensors, the assembled result compared with the unsharded one
@@ -650,7 +684,14 @@ def main():
     ap.add_argument("--no-strong", action="store_true", help="skip the strong-scaling leg (N>1)")
     ap.add_argument("--no-corr25", dest="corr25", action="store_false",
                     help="skip the 25 km all-pairs correlation probe (second half of BASELINE.json's metric)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the forecasts and GP records of the last timed step to DIR/<name>.npy (float64; "
+                         "with N > 1 every rank writes its own members as rank<r>.<name>.npy)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what this repo's CUDA path computed: not with --impl reference")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     # stdout carries ONE JSON line: libraries that write to file descriptor 1 (NCCL prints its version banner there when
     # NCCL_DEBUG is set) are pointed at stderr, and the line goes to the real stdout

@@ -18,6 +18,9 @@ The oracle (`oracle/`) is run beside it on every GP problem and on a sample of t
 (asserted here), which pins the oracle at full size too; its per-problem `sigma_f / nlml / n_pred` (values the
 reference computes but does not return) are stored as well.
 
+Node series (`anom`, float64 and nearly incompressible) are stored in full only for the networks of ANOM_YEARS
+(`anom_jobs`), so that each fixture stays under 1 MB; every network keeps its per-area sum of squares (`anom_sumsq`,
+aligned with `V_keys`) and its largest |value| (`anom_absmax`).
 Inputs are NOT stored: they are regenerated from seeds by bench.make_workload*; `input_sha256` guards the generators.
 Nothing is copied from the reference: functions are parsed out of the files where they lie and exec'd.
 """
@@ -49,6 +52,8 @@ from seaiceextentforecasting_b200.config import CONFIGS, RULE_ALL, RULE_POS, RUL
 REF = mg.REF
 FMIN, FMAX = bench.FMIN, bench.FMAX
 SCRIPTS = {name: rel for name, (rel, _, _) in mg.SWEEPS.items()}
+# windows T = 7, 9, 21, 32, 42 (short to full length), incl. the networks tests/test_bench_golden_gpu.py rebuilds on the CPU
+ANOM_YEARS = (1985, 1987, 1999, 2010, 2020)
 _TAU_LOG = []
 _orig_intra = mg.REFCN.Network.intra_links
 
@@ -230,7 +235,11 @@ def make(kind, procs):
     out["V_keys"] = np.concatenate([nets[(t[1], t[2])]["keys"] for t in tasks]).astype(np.int32)
     out["V_lens"] = np.concatenate([nets[(t[1], t[2])]["lens"] for t in tasks]).astype(np.int32)
     out["V_cells"] = np.concatenate([nets[(t[1], t[2])]["cells"] for t in tasks]).astype(np.int16)
-    out["anom"] = np.concatenate([nets[(t[1], t[2])]["anom"].reshape(-1) for t in tasks])
+    anoms = [nets[(t[1], t[2])]["anom"] for t in tasks]
+    out["anom_sumsq"] = np.concatenate([(a * a).sum(axis=1) for a in anoms])
+    out["anom_absmax"] = np.array([np.abs(a).max() for a in anoms])
+    out["anom_jobs"] = np.array([j for j, t in enumerate(tasks) if t[2] in ANOM_YEARS], dtype=np.int32)
+    out["anom"] = np.concatenate([anoms[j].reshape(-1) for j in out["anom_jobs"]])
     fname = {"north0": "bench_north_m0.npz", "north1": "bench_north_m1.npz", "south": "bench_south_feb.npz"}[kind]
     np.savez_compressed(os.path.join(HERE, fname), **out)
     nfail = int(out["gp_failed"].sum())

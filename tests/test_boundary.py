@@ -3,6 +3,7 @@ the product never touches the oracle; struct layouts match the header.  No compu
 import ctypes
 import os
 import re
+import shutil
 import subprocess
 
 import numpy as np
@@ -28,16 +29,24 @@ def test_library_exports_every_declared_symbol(lib_built):
     assert _lib.load().sie_abi_version() == _lib.ABI_VERSION == 2
 
 
+def cuobjdump():
+    """The cuobjdump of the toolkit whose nvcc builds the library (it need not be on PATH); the one on PATH where that
+    nvcc is a wrapper outside the toolkit."""
+    from seaiceextentforecasting_b200 import build
+    beside = os.path.join(os.path.dirname(os.path.realpath(build._nvcc())), "cuobjdump")
+    return beside if os.path.exists(beside) else shutil.which("cuobjdump") or beside
+
+
 def test_library_is_sm100a_only(lib_built):
     from seaiceextentforecasting_b200 import _lib
-    out = subprocess.run(["cuobjdump", "-lelf", _lib.LIB_PATH], capture_output=True, text=True).stdout
+    out = subprocess.run([cuobjdump(), "-lelf", _lib.LIB_PATH], capture_output=True, text=True).stdout
     archs = set(re.findall(r"sm_(\d+a?)", out))
     assert archs == {"100a"}, archs
 
 
 def test_sass_has_dmma_and_bulk_copy(lib_built):
     from seaiceextentforecasting_b200 import _lib
-    sass = subprocess.run(["cuobjdump", "-sass", _lib.LIB_PATH], capture_output=True, text=True).stdout
+    sass = subprocess.run([cuobjdump(), "-sass", _lib.LIB_PATH], capture_output=True, text=True).stdout
     assert "DMMA.8x8x4" in sass          # FP64 tensor pipe in the correlation kernel
     assert "UBLKCP" in sass              # cp.async.bulk (TMA engine) operand staging
     assert "SYNCS" in sass               # mbarrier
