@@ -217,6 +217,16 @@ int sie_gp_hyper_grid(const SieGpProblem* prob, int P, const double* sig_grid, i
                       const double* anom_sst, const int32_t* n_areas_sst, int max_areas_sst, int Tstride_sst,
                       int max_pred, SieGpResult* out, void* scratch, size_t scratch_bytes, void* stream);
 
+/* Grid minimum of MLII per problem (type-II maximum likelihood on the grid).  grid [P][n_ell][n_sig] are records of
+ * sie_gp_hyper_grid over the problems prob[p] with l = ell_grid[i].  A point is admissible when info == 0 and nlml is
+ * finite.  best[p] = i*n_sig + j of the smallest admissible nlml; ties go to the smallest flat index (np.argmin over
+ * [n_ell][n_sig]).  best[p] = -1 when no point is admissible.  tuned[p] = prob[p] with ell/sig replaced by the
+ * selected pair (unchanged when best[p] = -1), ready for sie_gp_forecast.  Reads only nlml and info of the records;
+ * the result is bit-reproducible.  Enqueue only. */
+int sie_gp_grid_select(const SieGpResult* grid, const SieGpProblem* prob, int P,
+                       const double* ell_grid, int n_ell, const double* sig_grid, int n_sig,
+                       SieGpProblem* tuned, int32_t* best, void* stream);
+
 /* ---------------------------------------------------------------------------------------------
  * Ingest (SURVEY.md 8(f) rows 1 and 4: the steps immediately before the hot path).
  * Replaces: readNSIDC                                          north/September1st.py:72-139

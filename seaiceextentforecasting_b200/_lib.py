@@ -56,6 +56,7 @@ _SIGS = {
     "sie_regrid_linear": (C.c_int, [c_p, C.c_int, C.c_int, c_p, c_p, C.c_int, c_p, c_p]),
     "sie_gp_hyper_grid": (C.c_int, [c_p, C.c_int, c_p, C.c_int, c_p, c_p, c_p, C.c_int, C.c_int, c_p, c_p, C.c_int,
                                     C.c_int, C.c_int, c_p, c_p, c_sz, c_p]),
+    "sie_gp_grid_select": (C.c_int, [c_p, c_p, C.c_int, c_p, C.c_int, c_p, C.c_int, c_p, c_p, c_p]),
     "sie_debug_gp_phases": (C.c_int, [C.POINTER(C.c_ulonglong)]),       # profiling aid (tools/gp_phases.py)
 }
 

@@ -1041,6 +1041,42 @@ __global__ void __launch_bounds__(1024) k_gp_order(const SieGpProblem* __restric
   for (int p = threadIdx.x; p < P; p += blockDim.x) order[atomicAdd(&hist[bucket(p)], 1)] = p;
 }
 
+// Grid minimum of MLII per problem (sie_gp_grid_select).  One warp per problem; lanes stride over the n_ell * n_sig
+// records reading only nlml / info.  Each lane keeps the first of its smallest admissible values (its indices ascend),
+// then the (value, flat index) pairs are reduced lexicographically with shuffles -- an associative, commutative min, so
+// every lane ends with np.argmin's answer whatever the reduction order (-0.0 == 0.0 resolves to the smaller index).
+constexpr int SEL_WARPS = 8;
+constexpr int SEL_NONE = 0x7fffffff;
+__global__ void __launch_bounds__(SEL_WARPS * 32)
+k_gp_grid_select(const SieGpResult* __restrict__ grid, const SieGpProblem* __restrict__ prob, int P,
+                 const double* __restrict__ ell_grid, int n_ell, const double* __restrict__ sig_grid, int n_sig,
+                 SieGpProblem* __restrict__ tuned, int32_t* __restrict__ best) {
+  const int p = blockIdx.x * SEL_WARPS + (threadIdx.x >> 5);
+  const int lane = threadIdx.x & 31;
+  if (p >= P) return;                                  // whole warp: p is uniform across it
+  const int n = n_ell * n_sig;
+  const SieGpResult* g = grid + (size_t)p * n;
+  double bv = __longlong_as_double(0x7ff0000000000000LL);   // +inf: no admissible point seen
+  int bi = SEL_NONE;
+  for (int k = lane; k < n; k += 32) {
+    const double v = __ldg(&g[k].nlml);
+    const int info = __ldg(&g[k].info);
+    if (info == 0 && isfinite(v) && v < bv) { bv = v; bi = k; }
+  }
+#pragma unroll
+  for (int off = 16; off > 0; off >>= 1) {
+    const double ov = __shfl_xor_sync(0xffffffffu, bv, off);
+    const int oi = __shfl_xor_sync(0xffffffffu, bi, off);
+    if (ov < bv || (ov == bv && oi < bi)) { bv = ov; bi = oi; }
+  }
+  if (lane == 0) {
+    SieGpProblem t = prob[p];
+    if (bi != SEL_NONE) { t.ell = ell_grid[bi / n_sig]; t.sig = sig_grid[bi % n_sig]; }
+    tuned[p] = t;
+    best[p] = bi == SEL_NONE ? -1 : bi;
+  }
+}
+
 __host__ size_t gp_per_cta_bytes(int max_pred) {
   size_t d = (size_t)9 * max_pred * max_pred + (size_t)3 * MAXN * max_pred + (size_t)3 * max_pred + (size_t)MAXN * LDS;
   size_t bytes = d * sizeof(double) + (size_t)max_pred * sizeof(int);
@@ -1118,4 +1154,16 @@ extern "C" int sie_gp_hyper_grid(const SieGpProblem* prob, int P, const double* 
   SIE_CHECK_ARG(sig_grid && n_sig > 0, "sig_grid must hold n_sig > 0 values");
   return gp_launch(prob, P, y_all, anom_sic, n_areas_sic, max_areas_sic, Tstride_sic, anom_sst, n_areas_sst,
                    max_areas_sst, Tstride_sst, max_pred, out, scratch, scratch_bytes, sig_grid, n_sig, stream);
+}
+
+extern "C" int sie_gp_grid_select(const SieGpResult* grid, const SieGpProblem* prob, int P, const double* ell_grid,
+                                  int n_ell, const double* sig_grid, int n_sig, SieGpProblem* tuned, int32_t* best,
+                                  void* stream) {
+  SIE_CHECK_ARG(grid && prob && ell_grid && sig_grid && tuned && best, "null pointer");
+  SIE_CHECK_ARG(P > 0 && n_ell > 0 && n_sig > 0, "P, n_ell and n_sig must be positive");
+  SIE_CHECK_ARG((long long)n_ell * n_sig < SEL_NONE, "n_ell * n_sig must be below 2^31 - 1");
+  k_gp_grid_select<<<(P - 1) / SEL_WARPS + 1, SEL_WARPS * 32, 0, (cudaStream_t)stream>>>(
+      grid, prob, P, ell_grid, n_ell, sig_grid, n_sig, tuned, best);
+  SIE_CHECK_LAUNCH();
+  return SIE_OK;
 }

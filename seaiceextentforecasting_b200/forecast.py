@@ -136,6 +136,52 @@ class GpBatch:
         return self.out.cpu().numpy().view(GP_RESULT_DTYPE)
 
 
+_ELL_COL = GP_PROBLEM_DTYPE.fields["ell"][1] // 8        # `ell` as a float64 column of a problem record
+assert GP_PROBLEM_DTYPE.itemsize % 8 == 0 and GP_PROBLEM_DTYPE.fields["ell"][1] % 8 == 0
+
+
+def expand_problems(prob_dev, ell_dev, out):
+    """`out` (uint8 device buffer of P * n_ell problem records) <- np.repeat(prob, n_ell) with copy i of every problem
+    at l = ell_dev[i]: the problem list sie_gp_hyper_grid evaluates on an (l, sigma_n~) grid.  Built on the device from
+    the first P records of `prob_dev` by copies into the preallocated `out` (no host round trip, no allocation), so a
+    captured step replays it."""
+    isz = GP_PROBLEM_DTYPE.itemsize
+    nl = ell_dev.numel()
+    P = out.numel() // (isz * nl)
+    out.view(P, nl, isz).copy_(prob_dev[:P * isz].view(P, 1, isz).expand(P, nl, isz))
+    out.view(torch.float64).view(P, nl, isz // 8)[:, :, _ELL_COL].copy_(ell_dev.view(1, nl).expand(P, nl))
+
+
+def grid_select(grid_dev, prob_dev, P, ell_dev, sig_dev, tuned_dev, best_dev):
+    """sie_gp_grid_select on the current stream: best_dev [P] (int32) <- flat index i * n_sig + j of the smallest
+    admissible nlML of every problem's grid records grid_dev [P][n_ell][n_sig] (-1: none admissible), tuned_dev [P]
+    <- prob_dev with (l, sigma_n~) = (ell_dev[i], sig_dev[j])."""
+    rc = _lib.load().sie_gp_grid_select(_ptr(grid_dev), _ptr(prob_dev), int(P), _ptr(ell_dev), ell_dev.numel(),
+                                        _ptr(sig_dev), sig_dev.numel(), _ptr(tuned_dev), _ptr(best_dev), _stream())
+    _lib.check(rc, "sie_gp_grid_select")
+
+
+class _GridBuffers:
+    """Device buffers of one (ells x sigs) hyper-parameter grid over a sweep's P problems."""
+
+    def __init__(self, ells, sigs, P):
+        self.ells, self.sigs = ells, sigs
+        self.ell_dev, self.sig_dev = h2d(ells), h2d(sigs)
+        self.prob = torch.empty(P * len(ells) * GP_PROBLEM_DTYPE.itemsize, dtype=torch.uint8, device="cuda")
+        self.out = torch.empty(P * len(ells) * len(sigs) * GP_RESULT_DTYPE.itemsize, dtype=torch.uint8, device="cuda")
+        self.gp = None                # GpBatch of hyper_grid() (the whole problem list in one launch)
+
+
+# (l, sigma_n~) a tuned sweep forecast with, and the flat grid index i * n_sig + j they came from (-1: the script's own)
+SELECTION_DTYPE = np.dtype([("ell", "<f8"), ("sig", "<f8"), ("best", "<i4")])
+
+
+def selection_records(tuned, best):
+    sel = np.empty(len(best), dtype=SELECTION_DTYPE)
+    sel["ell"], sel["sig"], sel["best"] = tuned["ell"], tuned["sig"], best
+    return sel
+
+
 class _SeriesSet:
     """Node series of ONE network given as a dict (the reference's `dataset['anoms']`), packed the way GpBatch reads a
     NetworkBatch: anomaly [1][nA][n+1], n_areas [1]."""
@@ -358,20 +404,24 @@ class SweepPlan:
         self.prob_member = self.prob_member[perm]
         return splits
 
-    def assemble(self, raw, meta=None, member=None):
+    def assemble(self, raw, meta=None, member=None, selection=None):
         """-> {config: {region_fmean / _fvar / _fmean_rt: array(years)}} like the reference's GPR dict
         (June1st_retro.py:284-290, rounded to 3 d.p.), the un-rounded values under '<region>_raw_*'.
         `raw`/`meta`/`member` may be the concatenation over all ranks (after a gather).  With `members` > 1 the result
-        is a list of such dicts, one per ensemble member."""
+        is a list of such dicts, one per ensemble member.  `selection` (SELECTION_DTYPE, aligned with `raw`; tuned
+        sweeps): also '<region>_ell' / '_sig', the hyper-parameters each forecast used, and '<region>_grid_index', the
+        flat grid index they came from (-1: the script's own setting was kept)."""
         meta = self.prob_meta if meta is None else meta
         member = self.prob_member if member is None else np.asarray(member)
         raw = np.asarray(raw)
         if self.members > 1:
             marr = np.asarray(meta, dtype=np.int64).reshape(-1, 3)
-            return [self._assemble_one(raw[member == mm], marr[member == mm]) for mm in range(self.members)]
-        return self._assemble_one(raw, meta)
+            return [self._assemble_one(raw[member == mm], marr[member == mm],
+                                       None if selection is None else np.asarray(selection)[member == mm])
+                    for mm in range(self.members)]
+        return self._assemble_one(raw, meta, selection)
 
-    def _assemble_one(self, raw, meta):
+    def _assemble_one(self, raw, meta, selection=None):
         m = np.asarray(meta, dtype=np.int64).reshape(-1, 3)
         out = {}
         if m.shape[0] == 0:
@@ -391,10 +441,13 @@ class SweepPlan:
                 tr = self.sie_trend[reg][row]                        # (slope, intercept) of that year's window
                 line_last = (years - FIRST_YEAR) * tr[:, 0] + tr[:, 1]   # lineT[-1], June1st_retro.py:285-286
                 i = years - self.fmin
-                for key, val in (("_fmean", fmean[sel]), ("_fvar", fvar[sel]),
-                                 ("_fmean_rt", np.round(fmean[sel] + line_last, 3)),
-                                 ("_raw_fmean", fmean_raw[sel]), ("_raw_fvar", fvar_raw[sel]),
-                                 ("_raw_fmean_rt", fmean_raw[sel] + line_last)):
+                items = [("_fmean", fmean[sel]), ("_fvar", fvar[sel]), ("_fmean_rt", np.round(fmean[sel] + line_last, 3)),
+                         ("_raw_fmean", fmean_raw[sel]), ("_raw_fvar", fvar_raw[sel]),
+                         ("_raw_fmean_rt", fmean_raw[sel] + line_last)]
+                if selection is not None:
+                    items += [("_ell", selection["ell"][sel]), ("_sig", selection["sig"][sel]),
+                              ("_grid_index", selection["best"][sel])]
+                for key, val in items:
                     arr = g.setdefault(reg + key, np.full(len(self.years), np.nan))
                     arr[i] = val
         return out
@@ -424,10 +477,15 @@ class RetrospectiveSweep:
                  sic_fields is a list
     sie        : dict region -> (Tfull,) September (or target-month) extent
     psar / sst_lat : weights for intra_links (cell area for the polar grid, latitude grid for SST)
+    hyper_grid : None (every forecast at its script's (l, sigma_n~)) or (ells, sigs): tuned sweep -- every forecast at
+                 the minimum of MLII's nlML over the ells x sigs grid of its own problem (type-II maximum likelihood on
+                 the grid, the search north/June1st.py:210-211 / :259-262 sets up), chosen on the device within the step;
+                 a problem with no admissible grid point keeps its script's setting
     """
 
     def __init__(self, config_names, sic_fields, sie, fmin, fmax, psar, sst_field=None, sst_lat=None,
-                 significance=0.01, max_areas=None, max_pred=384, rank=0, world=1, wave_T=(12,), keep_R=True):
+                 significance=0.01, max_areas=None, max_pred=384, rank=0, world=1, wave_T=(12,), keep_R=True,
+                 hyper_grid=None):
         require_cuda()
         member_fields = list(sic_fields) if isinstance(sic_fields, (list, tuple)) else [sic_fields]
         self.members = len(member_fields)
@@ -518,6 +576,18 @@ class RetrospectiveSweep:
         # pinned staging buffers so every step pays a real host->device copy
         self._pin = {name: torch.from_numpy(np.ascontiguousarray(arr)).pin_memory()
                      for name, arr in self._host_inputs().items()}
+        self._h2d_done = None                  # event after the last enqueued copy out of self._pin (load_inputs)
+        self._grids = {}                       # (ells, sigs) -> _GridBuffers (hyper_grid() and the tuned step)
+        self.tune = None
+        self.selection = None                  # tuned mode: SELECTION_DTYPE [P] of the step last read back
+        if hyper_grid is not None:
+            ells, sigs = (np.ascontiguousarray(a, dtype=np.float64).reshape(-1) for a in hyper_grid)
+            if ells.size < 1 or sigs.size < 1 or self.P < 1:
+                raise ValueError("hyper_grid needs at least one l and one sigma_n~ value and a sweep with problems")
+            self.tune = self._grid_buffers(ells, sigs)
+            self._tuned = torch.empty(self.P * GP_PROBLEM_DTYPE.itemsize, dtype=torch.uint8, device="cuda")
+            self._best = torch.empty(self.P, dtype=torch.int32, device="cuda")
+            self._gp_tuned = {}                # GP launch range -> GpBatch of its grid (its scratch also serves the forecast)
 
     def _host_inputs(self):
         p = self.plan
@@ -532,7 +602,8 @@ class RetrospectiveSweep:
         return int(sum(t.numel() * t.element_size() for t in self._pin.values()))
 
     def d2h_bytes(self):
-        return int(self.P * GP_RESULT_DTYPE.itemsize)
+        sel = 0 if self.tune is None else self.P * (GP_PROBLEM_DTYPE.itemsize + 4)    # tuned problems + best
+        return int(self.P * GP_RESULT_DTYPE.itemsize + sel)
 
     def upload(self):
         """Host -> device copy of every input (pinned, async on the current stream) into device buffers that keep their
@@ -541,7 +612,42 @@ class RetrospectiveSweep:
             self.dev = {k: torch.empty_like(t, device="cuda") for k, t in self._pin.items()}
         for k, t in self._pin.items():
             self.dev[k].copy_(t, non_blocking=True)
+        self._h2d_done = torch.cuda.Event()
+        self._h2d_done.record()
         return self.dev
+
+    def load_inputs(self, sic_fields, sst_field=None):
+        """Replace the sweep's input fields (same shapes and member count as the constructor's) for the next upload():
+        an ensemble far larger than one device batch streams through the same device buffers batch by batch instead of
+        re-allocating them (the stored correlation matrices alone are ~29 GB for 8 north members).  Rewrites the pinned
+        host buffers in place once every copy still reading them has finished.  `sst_field` None keeps the current SST
+        inputs.  The node capacity stays the constructor's: a batch with more ocean cells raises in check_status()."""
+        member_fields = list(sic_fields) if isinstance(sic_fields, (list, tuple)) else [sic_fields]
+        if len(member_fields) != self.members:
+            raise ValueError(f"{len(member_fields)} members given, the sweep was built for {self.members}")
+        for mf in member_fields:
+            for c in self.cfgs:
+                if np.shape(mf[c.name]) != (self.X, self.Y, self.Tfull):
+                    raise ValueError(f"{c.name}: SIC field of shape {np.shape(mf[c.name])}, expected "
+                                     f"{(self.X, self.Y, self.Tfull)}")
+        sic = np.stack([np.ascontiguousarray(mf[c.name], dtype=np.float64).reshape(self.X * self.Y, self.Tfull)
+                        for mf in member_fields for c in self.cfgs])
+        sst = None
+        if self.use_sst and sst_field is not None:
+            sst_members = list(sst_field) if isinstance(sst_field, (list, tuple)) else [sst_field] * self.members
+            if len(sst_members) != self.members:
+                raise ValueError(f"{len(sst_members)} SST fields given, the sweep was built for {self.members} members")
+            if any(np.shape(f) != (self.Xs, self.Ys, self.Tfull) for f in sst_members):
+                raise ValueError(f"SST fields must have the shape {(self.Xs, self.Ys, self.Tfull)}")
+            sst = np.stack([np.ascontiguousarray(f, dtype=np.float64).reshape(self.Xs * self.Ys, self.Tfull)
+                            for f in sst_members])
+        if self._h2d_done is not None:
+            self._h2d_done.synchronize()
+        self.sic_host = sic
+        self._pin["sic"].numpy()[...] = sic
+        if sst is not None:
+            self.sst_host = sst
+            self._pin["sst"].numpy()[...] = sst
 
     def compute(self, marks=None, waves=None):
         """Enqueue the whole hot path on the current stream (no host sync).  `marks`: optional list that receives
@@ -587,13 +693,15 @@ class RetrospectiveSweep:
             mark(tag + ".intra_links")
 
         main = torch.cuda.current_stream()
+        if self.tune is not None:               # before any side stream forks from `main`
+            expand_problems(d["prob"], self.tune.ell_dev, self.tune.prob)
         if waves == 0:
             # fully serial on the current stream (per-stage timing: no other kernel shares the GPU with the timed stage)
             if self.sst is not None:
                 chain("sst", self.sst, d["sst"], d["sst_field_idx"], d["sst_T"], d["sst_rcrit"], d["lat"])
             chain("sic", self.sic, d["sic"], d["job_field"], d["job_T"], d["rcrit"], d["psar"])
             mark("gp.start")
-            self.gp.run(d["prob"], d["y"], self.sic, self.sst)
+            self._gp_run(self.gp, None, mark, "gp")
             mark("gp")
             return
         if not two:
@@ -609,7 +717,7 @@ class RetrospectiveSweep:
             if self.sst is not None:
                 main.wait_stream(self._side)
             mark("gp.start")
-            self.gp.run(d["prob"], d["y"], self.sic, self.sst)
+            self._gp_run(self.gp, None, mark, "gp")
             mark("gp")
             return
         nw = len(self.waves)
@@ -655,7 +763,7 @@ class RetrospectiveSweep:
                             st.wait_event(sdone[v])
                     mark(f"gp{w}.start")
                     gp = self.gp if w == 0 else self.gp_wave[w - 1]
-                    gp.run(d["prob"], d["y"], self.sic, self.sst, (pr[0], split), out=self.gp.out)
+                    self._gp_run(gp, (pr[0], split), mark, f"gp{w}")
                     mark(f"gp{w}")
             if pr[1] > split:
                 st = gp_streams[w][1]
@@ -665,11 +773,51 @@ class RetrospectiveSweep:
                         if sdone[v] is not None:
                             st.wait_event(sdone[v])
                     mark(f"gps{w}.start")
-                    self.gp_sst[w].run(d["prob"], d["y"], self.sic, self.sst, (split, pr[1]), out=self.gp.out)
+                    self._gp_run(self.gp_sst[w], (split, pr[1]), mark, f"gps{w}")
                     mark(f"gps{w}")
         for (s1, s2) in self._streams:          # the step is complete on `main` once every wave has finished
             main.wait_stream(s1)
             main.wait_stream(s2)
+
+    def _gp_run(self, gp, pr, mark, tag):
+        """One GP launch of the step on the current stream over problems pr = (p0, p1) (None: all), results into
+        self.gp.out.  Tuned sweep: sie_gp_hyper_grid over the range's expanded problems, sie_gp_grid_select, then
+        sie_gp_forecast of the selected problems -- three launches in stream order, no host sync."""
+        d = self.dev
+        if self.tune is None:
+            gp.run(d["prob"], d["y"], self.sic, self.sst, pr, out=self.gp.out)
+            return
+        p0, p1 = (0, self.P) if pr is None else (int(pr[0]), int(pr[1]))
+        g, nl, ns = self.tune, len(self.tune.ells), len(self.tune.sigs)
+        isz, osz = GP_PROBLEM_DTYPE.itemsize, GP_RESULT_DTYPE.itemsize
+        gx = self._gp_tuned.get((p0, p1))
+        if gx is None:                          # first (eager) step: allocated before any graph capture
+            gx = self._gp_tuned[(p0, p1)] = GpBatch((p1 - p0) * nl, max_pred=self.gp.max_pred)
+        grid = g.out[p0 * nl * ns * osz:]
+        gx.run_grid(g.prob[p0 * nl * isz:], g.sig_dev, ns, d["y"], self.sic, self.sst, grid)
+        mark(tag + ".grid")
+        grid_select(grid, d["prob"][p0 * isz:], p1 - p0, g.ell_dev, g.sig_dev, self._tuned[p0 * isz:], self._best[p0:])
+        gx.run(self._tuned, d["y"], self.sic, self.sst, (p0, p1), out=self.gp.out)
+
+    def _grid_buffers(self, ells, sigs):
+        key = (ells.tobytes(), sigs.tobytes())
+        if key not in self._grids:
+            self._grids[key] = _GridBuffers(ells, sigs, self.P)
+        return self._grids[key]
+
+    def grid_records(self):
+        """Tuned sweep: the grid records [P][n_ell][n_sig] of the last step (host; synchronises)."""
+        g = self.tune
+        return g.out.cpu().numpy().view(GP_RESULT_DTYPE).reshape(self.P, len(g.ells), len(g.sigs))
+
+    def best_index(self):
+        """Tuned sweep: flat grid index i * n_sig + j each problem of the last step forecast at, -1 where no grid point
+        was admissible and the script's own (l, sigma_n~) was kept (host int32 [P]; synchronises)."""
+        return self._best.cpu().numpy()
+
+    def tuned_problems(self):
+        """Tuned sweep: the problem records the last step forecast with (host GP_PROBLEM_DTYPE [P]; synchronises)."""
+        return self._tuned.cpu().numpy().view(GP_PROBLEM_DTYPE)
 
     def hyper_grid(self, ells=None, sigs=None):
         """BASELINE.json configs[4] on this member: every GP problem of the sweep (year x init x region) evaluated on
@@ -679,38 +827,40 @@ class RetrospectiveSweep:
         ells = np.logspace(-7, 2, 20) if ells is None else np.asarray(ells, dtype=np.float64)
         sigs = np.logspace(-3, 9, 20) if sigs is None else np.asarray(sigs, dtype=np.float64)
         nl, ns = len(ells), len(sigs)
-        if getattr(self, "_grid", None) is None or self._grid[0] != (nl, ns):
-            prob = np.repeat(self.plan.prob, nl)
-            gp = GpBatch(self.P * nl, max_pred=self.gp.max_pred)
-            out = torch.empty(self.P * nl * ns * GP_RESULT_DTYPE.itemsize, dtype=torch.uint8, device="cuda")
-            self._grid = ((nl, ns), gp, out, prob)
-        _, gp, out, prob = self._grid
-        prob["ell"] = np.tile(ells, self.P)
-        gp.run_grid(h2d(prob.view(np.uint8)), h2d(sigs), ns, self.dev["y"], self.sic, self.sst, out)
-        return out.cpu().numpy().view(GP_RESULT_DTYPE).reshape(self.P, nl, ns)
+        g = self._grid_buffers(ells, sigs)
+        if g.gp is None:
+            g.gp = GpBatch(self.P * nl, max_pred=self.gp.max_pred)
+        expand_problems(self.dev["prob"], g.ell_dev, g.prob)
+        g.gp.run_grid(g.prob, g.sig_dev, ns, self.dev["y"], self.sic, self.sst, g.out)
+        return g.out.cpu().numpy().view(GP_RESULT_DTYPE).reshape(self.P, nl, ns)
 
     def kernel_launches(self):
         """Kernels of libsie_b200 enqueued by one compute(): 12 per network batch (K1: 3, K2: 4, K3-K5: 2, K6: 3), per
-        wave, + 2 per GP batch."""
+        wave, + 2 per GP batch (tuned sweep: 5 -- grid 2, select 1, forecast 2)."""
+        per_gp = 2 if self.tune is None else 5
         if not self.multi_wave:
-            return 12 * (2 if self.use_sst else 1) + 2
+            return 12 * (2 if self.use_sst else 1) + per_gp
         n = 0
         for w, (jr, sr, pr) in enumerate(self.waves):
             split = self.psplit[w] if self.gp_sst else pr[1]
-            n += 12 * (jr[1] > jr[0]) + 12 * (self.use_sst and sr[1] > sr[0]) + 2 * (split > pr[0]) + 2 * (pr[1] > split)
+            n += 12 * (jr[1] > jr[0]) + 12 * (self.use_sst and sr[1] > sr[0]) + per_gp * (split > pr[0]) + \
+                per_gp * (pr[1] > split)
         return int(n)
 
     def download(self):
         """Device -> host read of the GP results (synchronises).  Raises if any network build or GP problem ran out of
-        the capacity this sweep was sized for (a silent NaN forecast would look like a reference failure)."""
+        the capacity this sweep was sized for (a silent NaN forecast would look like a reference failure).  Tuned
+        sweep: also reads the selected (l, sigma_n~) and grid indices into self.selection."""
         self.raw = self.gp.results()[:self.P]
         self.check_status(self.raw)
+        if self.tune is not None:
+            self.selection = selection_records(self.tuned_problems(), self.best_index())
         return self.raw
 
     def run(self):
         self.upload()
         self.compute()
-        return self.plan.assemble(self.download())
+        return self.plan.assemble(self.download(), selection=self.selection)
 
     def run_many(self, n):
         """Generator over `n` sweeps run back to back (a perturbed-input ensemble, bench.py's end-to-end loop): every
@@ -721,14 +871,20 @@ class RetrospectiveSweep:
         Yields the same dict as run() per step; `self.raw` holds the records of the step just yielded."""
         if getattr(self, "_pin_out", None) is None:
             self._pin_out = [torch.empty(self.gp.out.numel(), dtype=torch.uint8).pin_memory() for _ in range(2)]
+        if self.tune is not None and getattr(self, "_pin_sel", None) is None:
+            self._pin_sel = [(torch.empty(self._tuned.numel(), dtype=torch.uint8).pin_memory(),
+                              torch.empty(self.P, dtype=torch.int32).pin_memory()) for _ in range(2)]
         pending = None
 
-        def finish(ev, buf):
+        def finish(ev, buf, k):
             ev.synchronize()
             self.raw = buf.numpy().view(GP_RESULT_DTYPE)[:self.P].copy()    # the buffer is reused two steps later
             if (self.raw["info"] == -2).any():
                 self.check_status(self.raw)
-            return self.plan.assemble(self.raw)
+            if self.tune is not None:
+                tp, bp = self._pin_sel[k]
+                self.selection = selection_records(tp.numpy().view(GP_PROBLEM_DTYPE), bp.numpy())
+            return self.plan.assemble(self.raw, selection=self.selection)
 
         # inputs are double-buffered on the device: step i+1's host -> device copy runs on a copy stream while step i
         # computes (with CUDA-graph replay the captured step reads fixed addresses: single buffer, copy in stream order)
@@ -755,6 +911,7 @@ class RetrospectiveSweep:
                         devs[k][key].copy_(t, non_blocking=True)
                     ev = torch.cuda.Event()
                     ev.record(cs)
+                self._h2d_done = ev
                 return ev
 
             if n > 0:
@@ -774,11 +931,15 @@ class RetrospectiveSweep:
                 self.compute()
             buf = self._pin_out[i & 1]
             buf.copy_(self.gp.out, non_blocking=True)
+            if self.tune is not None:
+                tp, bp = self._pin_sel[i & 1]
+                tp.copy_(self._tuned, non_blocking=True)
+                bp.copy_(self._best, non_blocking=True)
             ev = torch.cuda.Event()
             ev.record()
             if pending is not None:
                 yield finish(*pending)
-            pending = (ev, buf)
+            pending = (ev, buf, i & 1)
         if pending is not None:
             yield finish(*pending)
         self.check_status()                    # every step ran the same inputs: one check of the job statuses suffices

@@ -139,7 +139,31 @@ def gather_records(plan, raw, group=None, device=None, raw_dev=None):
     return raw_all, key_all[:, :3], key_all[:, 3]
 
 
-def gather_results(plan, raw, group=None, device=None):
-    """Every rank's GP records -> the assembled GPR dict of the whole sweep (SweepPlan.assemble) on every rank."""
+def gather_selection(selection, group=None, device=None):
+    """Tensor all-gather of every rank's tuned-sweep selection (RetrospectiveSweep.selection: the (l, sigma_n~, grid
+    index) each of its problems was forecast with), concatenated in the rank order of gather_records, so that every
+    rank assembles the same tuned dict."""
+    sel = np.ascontiguousarray(selection)
+    if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1:
+        return sel
+    world = dist.get_world_size(group)
+    if device is None:
+        device = "cuda" if dist.get_backend(group) == "nccl" else "cpu"
+    isz = sel.dtype.itemsize
+    n = torch.tensor([len(sel)], dtype=torch.int64, device=device)
+    counts = [torch.zeros_like(n) for _ in range(world)]
+    dist.all_gather(counts, n, group=group)
+    counts = [int(c.item()) for c in counts]
+    pay = torch.zeros(max(max(counts), 1) * isz, dtype=torch.uint8, device=device)
+    pay[:len(sel) * isz] = torch.from_numpy(sel.view(np.uint8).reshape(-1).copy()).to(device)
+    pays = [torch.empty_like(pay) for _ in range(world)]
+    dist.all_gather(pays, pay, group=group)
+    return np.concatenate([p.cpu().numpy()[:c * isz].view(sel.dtype) for p, c in zip(pays, counts)])
+
+
+def gather_results(plan, raw, group=None, device=None, selection=None):
+    """Every rank's GP records -> the assembled GPR dict of the whole sweep (SweepPlan.assemble) on every rank.
+    `selection`: this rank's tuned-sweep selection (RetrospectiveSweep.selection), gathered alongside."""
     raw_all, meta, member = gather_records(plan, raw, group, device)
-    return plan.assemble(raw_all, meta, member)
+    sel_all = None if selection is None else gather_selection(selection, group, device)
+    return plan.assemble(raw_all, meta, member, selection=sel_all)
