@@ -227,6 +227,32 @@ int sie_gp_grid_select(const SieGpResult* grid, const SieGpProblem* prob, int P,
                        const double* ell_grid, int n_ell, const double* sig_grid, int n_sig,
                        SieGpProblem* tuned, int32_t* best, void* stream);
 
+/* Grid marginal of the forecast per problem: the average over the (l, sigma_n~) grid of every grid point's forecast,
+ * weighted by its marginal likelihood (the Bayesian completion of type-II maximum likelihood on the grid).
+ * grid [P][n_grid] are records of sie_gp_hyper_grid (as for sie_gp_grid_select, n_grid = n_ell * n_sig).
+ *   A    = {k : info_k == 0 and nlml_k finite} (sie_gp_grid_select's rule), m = min over A of nlml_k
+ *   e_k  = exp(m - nlml_k), S0 = sum_A e_k, w_k = e_k / S0: a uniform prior over the admissible grid points -- on the
+ *          reference's log-spaced grids, log-uniform in l and in sigma_n~.  nlml profiles sigma_f out (sigma_f =
+ *          y^T K~^-1 y / n at each point), so these are profile-likelihood weights.
+ *   out[p] = record argmax with fmean = sum w mu, fvar = sum w (v + (mu - fmean)^2) (law of total variance, second
+ *          pass) and nlml = m - log S0 + log|A| (-log of the grid-averaged marginal likelihood)
+ *   stats[p] = {ess = S0^2 / sum e^2, w_max = 1 / S0, n_admissible = |A|, argmax = sie_gp_grid_select's best}
+ *   quant [P][n_q]: quantiles of F(x) = sum w Phi((x - mu) / sqrt(v)) at the levels q [n_q] (0 < q < 1; a component
+ *          with v <= 0 is a point mass at mu), by bisection on [min(mu - 40 sqrt(v)), max(mu + 40 sqrt(v))] over the
+ *          points with w > 0, keeping F(lo) < q <= F(hi), at most 128 halvings; the result is hi
+ * With A empty: out[p] = record 0 with fmean, fvar and nlml NaN (info stays the record's, e.g. -1), stats = {NaN, NaN,
+ * 0, -1}, quantiles NaN.  n_q == 0: q and quant may be NULL.  One warp per problem, fixed-order reductions: the result
+ * is bit-reproducible.  Enqueue only. */
+typedef struct SieGpMarginal {
+  double ess;            /* effective number of grid points, S0^2 / sum e_k^2 */
+  double w_max;          /* largest posterior weight, 1 / S0 */
+  int32_t n_admissible;  /* |A| */
+  int32_t argmax;        /* flat index of the largest weight; -1 when A is empty */
+} SieGpMarginal;         /* 24 bytes */
+
+int sie_gp_grid_marginal(const SieGpResult* grid, int P, int n_grid, const double* q, int n_q,
+                         SieGpResult* out, SieGpMarginal* stats, double* quant, void* stream);
+
 /* ---------------------------------------------------------------------------------------------
  * Ingest (SURVEY.md 8(f) rows 1 and 4: the steps immediately before the hot path).
  * Replaces: readNSIDC                                          north/September1st.py:72-139

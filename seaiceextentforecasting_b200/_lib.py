@@ -31,6 +31,10 @@ class SieGpResult(C.Structure):
                 ("expm_s", c_i32), ("info", c_i32), ("cycles_total", C.c_int64), ("cycles_expm", C.c_int64)]
 
 
+class SieGpMarginal(C.Structure):
+    _fields_ = [("ess", C.c_double), ("w_max", C.c_double), ("n_admissible", c_i32), ("argmax", c_i32)]
+
+
 _SIGS = {
     "sie_abi_version": (C.c_int, []),
     "sie_last_error": (C.c_char_p, []),
@@ -57,6 +61,7 @@ _SIGS = {
     "sie_gp_hyper_grid": (C.c_int, [c_p, C.c_int, c_p, C.c_int, c_p, c_p, c_p, C.c_int, C.c_int, c_p, c_p, C.c_int,
                                     C.c_int, C.c_int, c_p, c_p, c_sz, c_p]),
     "sie_gp_grid_select": (C.c_int, [c_p, c_p, C.c_int, c_p, C.c_int, c_p, C.c_int, c_p, c_p, c_p]),
+    "sie_gp_grid_marginal": (C.c_int, [c_p, C.c_int, C.c_int, c_p, C.c_int, c_p, c_p, c_p, c_p]),
     "sie_debug_gp_phases": (C.c_int, [C.POINTER(C.c_ulonglong)]),       # profiling aid (tools/gp_phases.py)
 }
 

@@ -1041,12 +1041,33 @@ __global__ void __launch_bounds__(1024) k_gp_order(const SieGpProblem* __restric
   for (int p = threadIdx.x; p < P; p += blockDim.x) order[atomicAdd(&hist[bucket(p)], 1)] = p;
 }
 
-// Grid minimum of MLII per problem (sie_gp_grid_select).  One warp per problem; lanes stride over the n_ell * n_sig
-// records reading only nlml / info.  Each lane keeps the first of its smallest admissible values (its indices ascend),
-// then the (value, flat index) pairs are reduced lexicographically with shuffles -- an associative, commutative min, so
-// every lane ends with np.argmin's answer whatever the reduction order (-0.0 == 0.0 resolves to the smaller index).
+// Grid minimum of MLII per problem (sie_gp_grid_select, and the weight maximum of sie_gp_grid_marginal).  One warp per
+// problem; lanes stride over the n grid records reading only nlml / info.  Each lane keeps the first of its smallest
+// admissible values (its indices ascend), then the (value, flat index) pairs are reduced lexicographically with
+// shuffles -- an associative, commutative min, so every lane ends with np.argmin's answer whatever the reduction order
+// (-0.0 == 0.0 resolves to the smaller index).  bi = SEL_NONE, bv = +inf when no record is admissible.
 constexpr int SEL_WARPS = 8;
 constexpr int SEL_NONE = 0x7fffffff;
+__device__ __forceinline__ bool gp_grid_admissible(const SieGpResult* r, double& nlml) {
+  nlml = __ldg(&r->nlml);
+  return __ldg(&r->info) == 0 && isfinite(nlml);
+}
+__device__ __forceinline__ void gp_grid_argmin_warp(const SieGpResult* __restrict__ g, int n, int lane, double& bv,
+                                                    int& bi) {
+  bv = __longlong_as_double(0x7ff0000000000000LL);   // +inf: no admissible point seen
+  bi = SEL_NONE;
+  for (int k = lane; k < n; k += 32) {
+    double v;
+    if (gp_grid_admissible(&g[k], v) && v < bv) { bv = v; bi = k; }
+  }
+#pragma unroll
+  for (int off = 16; off > 0; off >>= 1) {
+    const double ov = __shfl_xor_sync(0xffffffffu, bv, off);
+    const int oi = __shfl_xor_sync(0xffffffffu, bi, off);
+    if (ov < bv || (ov == bv && oi < bi)) { bv = ov; bi = oi; }
+  }
+}
+
 __global__ void __launch_bounds__(SEL_WARPS * 32)
 k_gp_grid_select(const SieGpResult* __restrict__ grid, const SieGpProblem* __restrict__ prob, int P,
                  const double* __restrict__ ell_grid, int n_ell, const double* __restrict__ sig_grid, int n_sig,
@@ -1055,25 +1076,149 @@ k_gp_grid_select(const SieGpResult* __restrict__ grid, const SieGpProblem* __res
   const int lane = threadIdx.x & 31;
   if (p >= P) return;                                  // whole warp: p is uniform across it
   const int n = n_ell * n_sig;
-  const SieGpResult* g = grid + (size_t)p * n;
-  double bv = __longlong_as_double(0x7ff0000000000000LL);   // +inf: no admissible point seen
-  int bi = SEL_NONE;
-  for (int k = lane; k < n; k += 32) {
-    const double v = __ldg(&g[k].nlml);
-    const int info = __ldg(&g[k].info);
-    if (info == 0 && isfinite(v) && v < bv) { bv = v; bi = k; }
-  }
-#pragma unroll
-  for (int off = 16; off > 0; off >>= 1) {
-    const double ov = __shfl_xor_sync(0xffffffffu, bv, off);
-    const int oi = __shfl_xor_sync(0xffffffffu, bi, off);
-    if (ov < bv || (ov == bv && oi < bi)) { bv = ov; bi = oi; }
-  }
+  double bv;
+  int bi;
+  gp_grid_argmin_warp(grid + (size_t)p * n, n, lane, bv, bi);
   if (lane == 0) {
     SieGpProblem t = prob[p];
     if (bi != SEL_NONE) { t.ell = ell_grid[bi / n_sig]; t.sig = sig_grid[bi % n_sig]; }
     tuned[p] = t;
     best[p] = bi == SEL_NONE ? -1 : bi;
+  }
+}
+
+// Grid marginal of the forecast per problem (sie_gp_grid_marginal).  One warp per problem, like k_gp_grid_select:
+//   1. m = min admissible nlml and its flat index (gp_grid_argmin_warp: the argmax of the weights is grid_select's best)
+//   2. e_k = exp(m - nlml_k) (0 outside A, 1 at the minimum), S0 = sum e, sum e^2, sum e mu, |A|
+//   3. fvar = sum e (v + (mu - fmean)^2) / S0 (second pass over the centred means)
+//   4. quantiles of the mixture CDF by bisection, F evaluated by the whole warp
+// Every sum is a per-lane sum over k = lane, lane + 32, ... (fixed order) followed by a fixed xor-shuffle tree; IEEE
+// addition commutes, so all 32 lanes hold the same bits and every branch on a reduced value is warp-uniform.  The
+// (e, mu, sd) of up to MARG_STAGE grid points are staged in shared memory for the bisection; a larger grid recomputes
+// them from the records at each step, with the same arithmetic, so both give the same bits.
+constexpr int MARG_WARPS = 4;
+constexpr int MARG_STAGE = 500;     // 4 warps x 500 points x 3 doubles = 48000 B of static shared memory per CTA
+
+__device__ __forceinline__ double warp_sum_xor(double v) {
+#pragma unroll
+  for (int off = 16; off > 0; off >>= 1) v = __dadd_rn(v, __shfl_xor_sync(0xffffffffu, v, off));
+  return v;
+}
+
+// Component k of the mixture: weight e (0 when k is not admissible or its weight underflows), mean, standard deviation
+// (0: v <= 0, a point mass at mu).  Reads fmean / fvar only for admissible points.
+__device__ __forceinline__ bool marg_component(const SieGpResult* __restrict__ r, double m, double& e, double& mu,
+                                               double& sd) {
+  double v;
+  e = 0.0; mu = 0.0; sd = 0.0;
+  if (!gp_grid_admissible(r, v)) return false;
+  e = exp(m - v);
+  mu = __ldg(&r->fmean);
+  const double var = __ldg(&r->fvar);
+  sd = var > 0.0 ? sqrt(var) : 0.0;
+  return true;
+}
+
+__global__ void __launch_bounds__(MARG_WARPS * 32)
+k_gp_grid_marginal(const SieGpResult* __restrict__ grid, int P, int n, const double* __restrict__ q, int n_q,
+                   SieGpResult* __restrict__ out, SieGpMarginal* __restrict__ stats, double* __restrict__ quant) {
+  __shared__ double s_e[MARG_WARPS][MARG_STAGE], s_mu[MARG_WARPS][MARG_STAGE], s_sd[MARG_WARPS][MARG_STAGE];
+  const int wp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int p = blockIdx.x * MARG_WARPS + wp;
+  if (p >= P) return;                                  // whole warp: p is uniform across it
+  const SieGpResult* g = grid + (size_t)p * n;
+  double m;
+  int bi;
+  gp_grid_argmin_warp(g, n, lane, m, bi);
+  if (bi == SEL_NONE) {                                // A empty: record 0 (its info says why), NaN moments / quantiles
+    if (lane == 0) {
+      SieGpResult r = g[0];
+      r.fmean = r.fvar = r.nlml = sie_nan();
+      out[p] = r;
+      SieGpMarginal s;
+      s.ess = s.w_max = sie_nan();
+      s.n_admissible = 0;
+      s.argmax = -1;
+      stats[p] = s;
+    }
+    for (int i = lane; i < n_q; i += 32) quant[(size_t)p * n_q + i] = sie_nan();
+    return;
+  }
+  const bool staged = n <= MARG_STAGE;
+  double s0 = 0.0, s2 = 0.0, s1 = 0.0, lo = __longlong_as_double(0x7ff0000000000000LL), hi = -lo;
+  int cnt = 0;
+  for (int k = lane; k < n; k += 32) {
+    double e, mu, sd;
+    cnt += marg_component(&g[k], m, e, mu, sd) ? 1 : 0;
+    if (staged) { s_e[wp][k] = e; s_mu[wp][k] = mu; s_sd[wp][k] = sd; }
+    if (e > 0.0) {
+      s0 = __dadd_rn(s0, e);
+      s2 = __fma_rn(e, e, s2);
+      s1 = __fma_rn(e, mu, s1);
+      lo = fmin(lo, mu - 40.0 * sd);
+      hi = fmax(hi, mu + 40.0 * sd);
+    }
+  }
+  s0 = warp_sum_xor(s0);
+  s2 = warp_sum_xor(s2);
+  s1 = warp_sum_xor(s1);
+#pragma unroll
+  for (int off = 16; off > 0; off >>= 1) {
+    cnt += __shfl_xor_sync(0xffffffffu, cnt, off);
+    lo = fmin(lo, __shfl_xor_sync(0xffffffffu, lo, off));
+    hi = fmax(hi, __shfl_xor_sync(0xffffffffu, hi, off));
+  }
+  const double fmean = s1 / s0;
+  double sv = 0.0;
+  for (int k = lane; k < n; k += 32) {
+    double v;
+    if (gp_grid_admissible(&g[k], v)) {
+      const double e = exp(m - v);
+      if (e > 0.0) {
+        const double d = __ldg(&g[k].fmean) - fmean;
+        sv = __fma_rn(e, __fma_rn(d, d, __ldg(&g[k].fvar)), sv);
+      }
+    }
+  }
+  sv = warp_sum_xor(sv);
+  __syncwarp();                                        // the staged components are visible to the whole warp
+
+  // F(x) = sum_k e_k Phi((x - mu_k) / sd_k) / S0, a point mass (sd = 0) counting from x = mu on (right-continuous)
+  auto cdf = [&](double x) {
+    double f = 0.0;
+    for (int k = lane; k < n; k += 32) {
+      double e, mu, sd;
+      if (staged) { e = s_e[wp][k]; mu = s_mu[wp][k]; sd = s_sd[wp][k]; }
+      else marg_component(&g[k], m, e, mu, sd);
+      if (e > 0.0) f = __fma_rn(e, sd > 0.0 ? normcdf((x - mu) / sd) : (x >= mu ? 1.0 : 0.0), f);
+    }
+    return warp_sum_xor(f) / s0;
+  };
+  for (int i = 0; i < n_q; ++i) {
+    const double t = q[i];
+    double a = lo, b = hi;
+    if (cdf(a) >= t) b = a;                            // a point mass at the lower end already holds q
+    else if (cdf(b) >= t) {                            // invariant F(a) < q <= F(b)
+      for (int it = 0; it < 128; ++it) {
+        const double c = 0.5 * a + 0.5 * b;
+        if (c == a || c == b) break;
+        if (cdf(c) >= t) b = c; else a = c;
+      }
+    }                                                  // else: sum w rounds below q; hi is the upper end
+    if (lane == 0) quant[(size_t)p * n_q + i] = b;
+  }
+  if (lane == 0) {
+    SieGpResult r = g[bi];
+    r.fmean = fmean;
+    r.fvar = sv / s0;
+    r.nlml = m - log(s0) + log((double)cnt);
+    out[p] = r;
+    SieGpMarginal s;
+    s.ess = s0 * s0 / s2;
+    s.w_max = 1.0 / s0;
+    s.n_admissible = cnt;
+    s.argmax = bi;
+    stats[p] = s;
   }
 }
 
@@ -1164,6 +1309,18 @@ extern "C" int sie_gp_grid_select(const SieGpResult* grid, const SieGpProblem* p
   SIE_CHECK_ARG((long long)n_ell * n_sig < SEL_NONE, "n_ell * n_sig must be below 2^31 - 1");
   k_gp_grid_select<<<(P - 1) / SEL_WARPS + 1, SEL_WARPS * 32, 0, (cudaStream_t)stream>>>(
       grid, prob, P, ell_grid, n_ell, sig_grid, n_sig, tuned, best);
+  SIE_CHECK_LAUNCH();
+  return SIE_OK;
+}
+
+extern "C" int sie_gp_grid_marginal(const SieGpResult* grid, int P, int n_grid, const double* q, int n_q,
+                                    SieGpResult* out, SieGpMarginal* stats, double* quant, void* stream) {
+  SIE_CHECK_ARG(grid && out && stats, "null pointer");
+  SIE_CHECK_ARG(P > 0 && n_grid > 0, "P and n_grid must be positive");
+  SIE_CHECK_ARG(n_q >= 0, "n_q must not be negative");
+  SIE_CHECK_ARG(n_q == 0 || (q && quant), "q and quant must not be null when n_q > 0");
+  k_gp_grid_marginal<<<(P - 1) / MARG_WARPS + 1, MARG_WARPS * 32, 0, (cudaStream_t)stream>>>(
+      grid, P, n_grid, q, n_q, out, stats, quant);
   SIE_CHECK_LAUNCH();
   return SIE_OK;
 }

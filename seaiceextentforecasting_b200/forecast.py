@@ -182,6 +182,49 @@ def selection_records(tuned, best):
     return sel
 
 
+# SieGpMarginal (include/sie_b200.h): what sie_gp_grid_marginal reports about each problem's grid posterior
+GP_MARGINAL_DTYPE = np.dtype([("ess", "<f8"), ("w_max", "<f8"), ("n_admissible", "<i4"), ("argmax", "<i4")])
+assert GP_MARGINAL_DTYPE.itemsize == C.sizeof(_lib.SieGpMarginal)
+DEFAULT_QUANTILES = (0.05, 0.5, 0.95)
+
+
+def marginal_dtype(n_q):
+    """Per-problem record of a marginalised forecast: GP_MARGINAL_DTYPE's fields plus `quantiles`, a float64 sub-array
+    of the n_q predictive quantiles (detrended).  Its length is the number of levels, hence a function of n_q."""
+    return np.dtype(GP_MARGINAL_DTYPE.descr + [("quantiles", "<f8", (int(n_q),))])
+
+
+def marginal_records(stats, quant):
+    """stats: GP_MARGINAL_DTYPE [P] (or its bytes), quant: float64 [P][n_q] -> marginal_dtype(n_q) [P]."""
+    stats = np.asarray(stats).view(GP_MARGINAL_DTYPE).reshape(-1)
+    quant = np.asarray(quant, dtype=np.float64).reshape(-1)
+    quant = quant.reshape(len(stats), quant.size // max(1, len(stats)))
+    rec = np.empty(len(stats), dtype=marginal_dtype(quant.shape[1]))
+    for f in GP_MARGINAL_DTYPE.names:
+        rec[f] = stats[f]
+    rec["quantiles"] = quant
+    return rec
+
+
+def check_levels(quantiles):
+    """-> the quantile levels as float64; raises ValueError unless every level lies strictly inside (0, 1)."""
+    q = np.ascontiguousarray(quantiles, dtype=np.float64).reshape(-1)
+    if not np.all((q > 0.0) & (q < 1.0)):
+        raise ValueError(f"quantile levels must lie strictly between 0 and 1, got {q.tolist()}")
+    return q
+
+
+def grid_marginal(grid_dev, P, n_grid, q_dev, out_dev, stats_dev, quant_dev):
+    """sie_gp_grid_marginal on the current stream: out_dev [P] (GP records) <- the marginal-likelihood-weighted mixture
+    of every problem's grid records grid_dev [P][n_grid], stats_dev [P] (GP_MARGINAL_DTYPE) <- ESS, largest weight,
+    |A| and its index, quant_dev [P][n_q] <- the mixture's quantiles at the levels q_dev [n_q] (q_dev None: none)."""
+    n_q = 0 if q_dev is None else q_dev.numel()
+    null = C.c_void_p(0)
+    rc = _lib.load().sie_gp_grid_marginal(_ptr(grid_dev), int(P), int(n_grid), _ptr(q_dev) if n_q else null, n_q,
+                                          _ptr(out_dev), _ptr(stats_dev), _ptr(quant_dev) if n_q else null, _stream())
+    _lib.check(rc, "sie_gp_grid_marginal")
+
+
 class _SeriesSet:
     """Node series of ONE network given as a dict (the reference's `dataset['anoms']`), packed the way GpBatch reads a
     NetworkBatch: anomaly [1][nA][n+1], n_areas [1]."""
@@ -226,11 +269,9 @@ def forecast(y, anoms_sic, anoms_sst=None, rule=0, alpha=0.05, zscore=False, ell
     return gp.results()[0]
 
 
-def hyper_grid(y, anoms_sic, anoms_sst=None, rule=0, alpha=0.05, zscore=False, ells=None, sigs=None, want_grad=False):
-    """Grid search over the reference's hyper-parameter grids `ls = np.logspace(-7,2,20)`, `ss = np.logspace(-3,9,20)`
-    (north/June1st.py:210-211; the `minimize(MLII, ...)` call at :259-262 is commented out there): negative log marginal
-    likelihood of MLII() for every (l, sigma_n~) pair, one expm per l.
-    Returns (records [len(ells)][len(sigs)], (i, j) of the smallest finite nlML)."""
+def _grid_on_device(y, anoms_sic, anoms_sst, rule, alpha, zscore, ells, sigs, want_grad):
+    """One problem's (l, sigma_n~) grid records, left on the device: (uint8 buffer of [len(ells)][len(sigs)] records,
+    ells, sigs); ells / sigs None are the reference's grids."""
     require_cuda()
     ells = np.logspace(-7, 2, 20) if ells is None else np.asarray(ells, dtype=np.float64)
     sigs = np.logspace(-3, 9, 20) if sigs is None else np.asarray(sigs, dtype=np.float64)
@@ -244,10 +285,36 @@ def hyper_grid(y, anoms_sic, anoms_sst=None, rule=0, alpha=0.05, zscore=False, e
     gp = GpBatch(len(ells), max_pred=max(4, npred))
     out = torch.empty(len(ells) * len(sigs) * GP_RESULT_DTYPE.itemsize, dtype=torch.uint8, device="cuda")
     gp.run_grid(h2d(prob.view(np.uint8)), h2d(sigs), len(sigs), h2d(y), s1, s2, out)
+    return out, ells, sigs
+
+
+def hyper_grid(y, anoms_sic, anoms_sst=None, rule=0, alpha=0.05, zscore=False, ells=None, sigs=None, want_grad=False):
+    """Grid search over the reference's hyper-parameter grids `ls = np.logspace(-7,2,20)`, `ss = np.logspace(-3,9,20)`
+    (north/June1st.py:210-211; the `minimize(MLII, ...)` call at :259-262 is commented out there): negative log marginal
+    likelihood of MLII() for every (l, sigma_n~) pair, one expm per l.
+    Returns (records [len(ells)][len(sigs)], (i, j) of the smallest finite nlML)."""
+    out, ells, sigs = _grid_on_device(y, anoms_sic, anoms_sst, rule, alpha, zscore, ells, sigs, want_grad)
     rec = out.cpu().numpy().view(GP_RESULT_DTYPE).reshape(len(ells), len(sigs))
     nl = np.where((rec["info"] == 0) & np.isfinite(rec["nlml"]), rec["nlml"], np.inf)
     best = np.unravel_index(int(np.argmin(nl)), nl.shape)
     return rec, (int(best[0]), int(best[1]))
+
+
+def marginal_forecast(y, anoms_sic, anoms_sst=None, rule=0, alpha=0.05, zscore=False, ells=None, sigs=None,
+                      quantiles=DEFAULT_QUANTILES):
+    """The forecast averaged over the (l, sigma_n~) grid (hyper_grid's problem and grids), every grid point weighted by
+    its marginal likelihood, on the device (sie_gp_grid_marginal).  Returns (record, stats, quantiles): the GP record
+    with the mixture's fmean / fvar and nlml = -log of the grid-averaged marginal likelihood (the other fields are the
+    largest-weight point's), GP_MARGINAL_DTYPE stats (ESS, largest weight, |A|, its flat index), and the mixture's
+    predictive quantiles at `quantiles` (detrended; NaN where no grid point is admissible)."""
+    q = check_levels(quantiles)
+    out, ells, sigs = _grid_on_device(y, anoms_sic, anoms_sst, rule, alpha, zscore, ells, sigs, False)
+    rec = torch.empty(GP_RESULT_DTYPE.itemsize, dtype=torch.uint8, device="cuda")
+    stats = torch.empty(GP_MARGINAL_DTYPE.itemsize, dtype=torch.uint8, device="cuda")
+    quant = torch.empty(max(1, q.size), dtype=torch.float64, device="cuda")
+    grid_marginal(out, 1, len(ells) * len(sigs), h2d(q) if q.size else None, rec, stats, quant)
+    return (rec.cpu().numpy().view(GP_RESULT_DTYPE)[0], stats.cpu().numpy().view(GP_MARGINAL_DTYPE)[0],
+            quant.cpu().numpy()[:q.size])
 
 
 def mlii(theta, y, anoms_sic, anoms_sst=None, rule=0, alpha=0.05, zscore=False):
@@ -404,24 +471,28 @@ class SweepPlan:
         self.prob_member = self.prob_member[perm]
         return splits
 
-    def assemble(self, raw, meta=None, member=None, selection=None):
+    def assemble(self, raw, meta=None, member=None, selection=None, marginal=None):
         """-> {config: {region_fmean / _fvar / _fmean_rt: array(years)}} like the reference's GPR dict
         (June1st_retro.py:284-290, rounded to 3 d.p.), the un-rounded values under '<region>_raw_*'.
         `raw`/`meta`/`member` may be the concatenation over all ranks (after a gather).  With `members` > 1 the result
         is a list of such dicts, one per ensemble member.  `selection` (SELECTION_DTYPE, aligned with `raw`; tuned
         sweeps): also '<region>_ell' / '_sig', the hyper-parameters each forecast used, and '<region>_grid_index', the
-        flat grid index they came from (-1: the script's own setting was kept)."""
+        flat grid index they came from (-1: the script's own setting was kept).  `marginal` (marginal_dtype(n_q),
+        aligned with `raw`; marginalised sweeps): also '<region>_grid_index' (the largest-weight grid point, -1: none
+        admissible), '_ess', '_w_max', '_quantiles' (array(years, n_q), detrended) and '_quantiles_rt' (the same
+        re-trended like '_raw_fmean_rt')."""
         meta = self.prob_meta if meta is None else meta
         member = self.prob_member if member is None else np.asarray(member)
         raw = np.asarray(raw)
         if self.members > 1:
             marr = np.asarray(meta, dtype=np.int64).reshape(-1, 3)
             return [self._assemble_one(raw[member == mm], marr[member == mm],
-                                       None if selection is None else np.asarray(selection)[member == mm])
+                                       None if selection is None else np.asarray(selection)[member == mm],
+                                       None if marginal is None else np.asarray(marginal)[member == mm])
                     for mm in range(self.members)]
-        return self._assemble_one(raw, meta, selection)
+        return self._assemble_one(raw, meta, selection, marginal)
 
-    def _assemble_one(self, raw, meta, selection=None):
+    def _assemble_one(self, raw, meta, selection=None, marginal=None):
         m = np.asarray(meta, dtype=np.int64).reshape(-1, 3)
         out = {}
         if m.shape[0] == 0:
@@ -447,8 +518,13 @@ class SweepPlan:
                 if selection is not None:
                     items += [("_ell", selection["ell"][sel]), ("_sig", selection["sig"][sel]),
                               ("_grid_index", selection["best"][sel])]
+                if marginal is not None:
+                    qs = marginal["quantiles"][sel]
+                    items += [("_grid_index", marginal["argmax"][sel]), ("_ess", marginal["ess"][sel]),
+                              ("_w_max", marginal["w_max"][sel]), ("_quantiles", qs),
+                              ("_quantiles_rt", qs + line_last[:, None])]
                 for key, val in items:
-                    arr = g.setdefault(reg + key, np.full(len(self.years), np.nan))
+                    arr = g.setdefault(reg + key, np.full((len(self.years),) + np.shape(val)[1:], np.nan))
                     arr[i] = val
         return out
 
@@ -481,11 +557,25 @@ class RetrospectiveSweep:
                  the minimum of MLII's nlML over the ells x sigs grid of its own problem (type-II maximum likelihood on
                  the grid, the search north/June1st.py:210-211 / :259-262 sets up), chosen on the device within the step;
                  a problem with no admissible grid point keeps its script's setting
+    hyper_mode : with hyper_grid: "argmin" (the default: the tuned sweep above) or "marginal" -- every forecast is the
+                 average of its problem's forecasts at all grid points, each weighted by its marginal likelihood
+                 (sie_gp_grid_marginal: a uniform prior over the admissible grid points; the variance includes the
+                 spread of the grid means); the step runs the grid and that one reduction, no second forecast
+    quantiles  : marginal mode: levels in (0, 1) of the predictive quantiles to compute from each forecast's mixture
+                 (self.marginal["quantiles"], '<region>_quantiles' of the assembled dict)
     """
 
     def __init__(self, config_names, sic_fields, sie, fmin, fmax, psar, sst_field=None, sst_lat=None,
                  significance=0.01, max_areas=None, max_pred=384, rank=0, world=1, wave_T=(12,), keep_R=True,
-                 hyper_grid=None):
+                 hyper_grid=None, hyper_mode=None, quantiles=()):
+        if hyper_mode is not None and hyper_grid is None:
+            raise ValueError("hyper_mode needs a hyper_grid")
+        hyper_mode = "argmin" if hyper_mode is None else hyper_mode
+        if hyper_mode not in ("argmin", "marginal"):
+            raise ValueError(f"hyper_mode must be 'argmin' or 'marginal', got {hyper_mode!r}")
+        levels = check_levels(quantiles)
+        if levels.size and hyper_mode != "marginal":
+            raise ValueError("quantiles are computed by marginal sweeps only (hyper_mode='marginal')")
         require_cuda()
         member_fields = list(sic_fields) if isinstance(sic_fields, (list, tuple)) else [sic_fields]
         self.members = len(member_fields)
@@ -579,14 +669,22 @@ class RetrospectiveSweep:
         self._h2d_done = None                  # event after the last enqueued copy out of self._pin (load_inputs)
         self._grids = {}                       # (ells, sigs) -> _GridBuffers (hyper_grid() and the tuned step)
         self.tune = None
+        self.hyper_mode = hyper_mode if hyper_grid is not None else None
+        self.levels = levels
         self.selection = None                  # tuned mode: SELECTION_DTYPE [P] of the step last read back
+        self.marginal = None                   # marginal mode: marginal_dtype(n_q) [P] of the step last read back
         if hyper_grid is not None:
             ells, sigs = (np.ascontiguousarray(a, dtype=np.float64).reshape(-1) for a in hyper_grid)
             if ells.size < 1 or sigs.size < 1 or self.P < 1:
                 raise ValueError("hyper_grid needs at least one l and one sigma_n~ value and a sweep with problems")
             self.tune = self._grid_buffers(ells, sigs)
-            self._tuned = torch.empty(self.P * GP_PROBLEM_DTYPE.itemsize, dtype=torch.uint8, device="cuda")
-            self._best = torch.empty(self.P, dtype=torch.int32, device="cuda")
+            if hyper_mode == "argmin":
+                self._tuned = torch.empty(self.P * GP_PROBLEM_DTYPE.itemsize, dtype=torch.uint8, device="cuda")
+                self._best = torch.empty(self.P, dtype=torch.int32, device="cuda")
+            else:
+                self._q_dev = h2d(levels) if levels.size else None
+                self._mstats = torch.empty(self.P * GP_MARGINAL_DTYPE.itemsize, dtype=torch.uint8, device="cuda")
+                self._quant = torch.empty(max(1, self.P * levels.size), dtype=torch.float64, device="cuda")
             self._gp_tuned = {}                # GP launch range -> GpBatch of its grid (its scratch also serves the forecast)
 
     def _host_inputs(self):
@@ -602,7 +700,12 @@ class RetrospectiveSweep:
         return int(sum(t.numel() * t.element_size() for t in self._pin.values()))
 
     def d2h_bytes(self):
-        sel = 0 if self.tune is None else self.P * (GP_PROBLEM_DTYPE.itemsize + 4)    # tuned problems + best
+        if self.tune is None:
+            sel = 0
+        elif self.hyper_mode == "argmin":
+            sel = self.P * (GP_PROBLEM_DTYPE.itemsize + 4)                      # tuned problems + best
+        else:
+            sel = self.P * (GP_MARGINAL_DTYPE.itemsize + 8 * self.levels.size)  # stats + quantiles
         return int(self.P * GP_RESULT_DTYPE.itemsize + sel)
 
     def upload(self):
@@ -782,7 +885,8 @@ class RetrospectiveSweep:
     def _gp_run(self, gp, pr, mark, tag):
         """One GP launch of the step on the current stream over problems pr = (p0, p1) (None: all), results into
         self.gp.out.  Tuned sweep: sie_gp_hyper_grid over the range's expanded problems, sie_gp_grid_select, then
-        sie_gp_forecast of the selected problems -- three launches in stream order, no host sync."""
+        sie_gp_forecast of the selected problems -- three launches in stream order, no host sync.  Marginal sweep: the
+        grid, then sie_gp_grid_marginal straight into self.gp.out and the range's stats / quantiles."""
         d = self.dev
         if self.tune is None:
             gp.run(d["prob"], d["y"], self.sic, self.sst, pr, out=self.gp.out)
@@ -796,6 +900,11 @@ class RetrospectiveSweep:
         grid = g.out[p0 * nl * ns * osz:]
         gx.run_grid(g.prob[p0 * nl * isz:], g.sig_dev, ns, d["y"], self.sic, self.sst, grid)
         mark(tag + ".grid")
+        if self.hyper_mode == "marginal":
+            nq = self.levels.size
+            grid_marginal(grid, p1 - p0, nl * ns, self._q_dev, self.gp.out[p0 * osz:],
+                          self._mstats[p0 * GP_MARGINAL_DTYPE.itemsize:], self._quant[p0 * nq:])
+            return
         grid_select(grid, d["prob"][p0 * isz:], p1 - p0, g.ell_dev, g.sig_dev, self._tuned[p0 * isz:], self._best[p0:])
         gx.run(self._tuned, d["y"], self.sic, self.sst, (p0, p1), out=self.gp.out)
 
@@ -836,8 +945,9 @@ class RetrospectiveSweep:
 
     def kernel_launches(self):
         """Kernels of libsie_b200 enqueued by one compute(): 12 per network batch (K1: 3, K2: 4, K3-K5: 2, K6: 3), per
-        wave, + 2 per GP batch (tuned sweep: 5 -- grid 2, select 1, forecast 2)."""
-        per_gp = 2 if self.tune is None else 5
+        wave, + 2 per GP batch (tuned sweep: 5 -- grid 2, select 1, forecast 2; marginal sweep: 3 -- grid 2,
+        marginal 1)."""
+        per_gp = 2 if self.tune is None else (5 if self.hyper_mode == "argmin" else 3)
         if not self.multi_wave:
             return 12 * (2 if self.use_sst else 1) + per_gp
         n = 0
@@ -850,17 +960,21 @@ class RetrospectiveSweep:
     def download(self):
         """Device -> host read of the GP results (synchronises).  Raises if any network build or GP problem ran out of
         the capacity this sweep was sized for (a silent NaN forecast would look like a reference failure).  Tuned
-        sweep: also reads the selected (l, sigma_n~) and grid indices into self.selection."""
+        sweep: also reads the selected (l, sigma_n~) and grid indices into self.selection; marginal sweep: the grid
+        posterior's stats and the quantiles into self.marginal."""
         self.raw = self.gp.results()[:self.P]
         self.check_status(self.raw)
-        if self.tune is not None:
+        if self.hyper_mode == "argmin":
             self.selection = selection_records(self.tuned_problems(), self.best_index())
+        elif self.hyper_mode == "marginal":
+            self.marginal = marginal_records(self._mstats.cpu().numpy(),
+                                             self._quant.cpu().numpy()[:self.P * self.levels.size])
         return self.raw
 
     def run(self):
         self.upload()
         self.compute()
-        return self.plan.assemble(self.download(), selection=self.selection)
+        return self.plan.assemble(self.download(), selection=self.selection, marginal=self.marginal)
 
     def run_many(self, n):
         """Generator over `n` sweeps run back to back (a perturbed-input ensemble, bench.py's end-to-end loop): every
@@ -871,9 +985,12 @@ class RetrospectiveSweep:
         Yields the same dict as run() per step; `self.raw` holds the records of the step just yielded."""
         if getattr(self, "_pin_out", None) is None:
             self._pin_out = [torch.empty(self.gp.out.numel(), dtype=torch.uint8).pin_memory() for _ in range(2)]
-        if self.tune is not None and getattr(self, "_pin_sel", None) is None:
+        if self.hyper_mode == "argmin" and getattr(self, "_pin_sel", None) is None:
             self._pin_sel = [(torch.empty(self._tuned.numel(), dtype=torch.uint8).pin_memory(),
                               torch.empty(self.P, dtype=torch.int32).pin_memory()) for _ in range(2)]
+        if self.hyper_mode == "marginal" and getattr(self, "_pin_marg", None) is None:
+            self._pin_marg = [(torch.empty(self._mstats.numel(), dtype=torch.uint8).pin_memory(),
+                               torch.empty(self._quant.numel(), dtype=torch.float64).pin_memory()) for _ in range(2)]
         pending = None
 
         def finish(ev, buf, k):
@@ -881,10 +998,13 @@ class RetrospectiveSweep:
             self.raw = buf.numpy().view(GP_RESULT_DTYPE)[:self.P].copy()    # the buffer is reused two steps later
             if (self.raw["info"] == -2).any():
                 self.check_status(self.raw)
-            if self.tune is not None:
+            if self.hyper_mode == "argmin":
                 tp, bp = self._pin_sel[k]
                 self.selection = selection_records(tp.numpy().view(GP_PROBLEM_DTYPE), bp.numpy())
-            return self.plan.assemble(self.raw, selection=self.selection)
+            elif self.hyper_mode == "marginal":
+                sp, qp = self._pin_marg[k]
+                self.marginal = marginal_records(sp.numpy(), qp.numpy()[:self.P * self.levels.size])
+            return self.plan.assemble(self.raw, selection=self.selection, marginal=self.marginal)
 
         # inputs are double-buffered on the device: step i+1's host -> device copy runs on a copy stream while step i
         # computes (with CUDA-graph replay the captured step reads fixed addresses: single buffer, copy in stream order)
@@ -931,10 +1051,14 @@ class RetrospectiveSweep:
                 self.compute()
             buf = self._pin_out[i & 1]
             buf.copy_(self.gp.out, non_blocking=True)
-            if self.tune is not None:
+            if self.hyper_mode == "argmin":
                 tp, bp = self._pin_sel[i & 1]
                 tp.copy_(self._tuned, non_blocking=True)
                 bp.copy_(self._best, non_blocking=True)
+            elif self.hyper_mode == "marginal":
+                sp, qp = self._pin_marg[i & 1]
+                sp.copy_(self._mstats, non_blocking=True)
+                qp.copy_(self._quant, non_blocking=True)
             ev = torch.cuda.Event()
             ev.record()
             if pending is not None:

@@ -142,7 +142,8 @@ def gather_records(plan, raw, group=None, device=None, raw_dev=None):
 def gather_selection(selection, group=None, device=None):
     """Tensor all-gather of every rank's tuned-sweep selection (RetrospectiveSweep.selection: the (l, sigma_n~, grid
     index) each of its problems was forecast with), concatenated in the rank order of gather_records, so that every
-    rank assembles the same tuned dict."""
+    rank assembles the same tuned dict.  Any structured per-problem array gathers the same way (the marginal records
+    of a marginalised sweep)."""
     sel = np.ascontiguousarray(selection)
     if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1:
         return sel
@@ -161,9 +162,11 @@ def gather_selection(selection, group=None, device=None):
     return np.concatenate([p.cpu().numpy()[:c * isz].view(sel.dtype) for p, c in zip(pays, counts)])
 
 
-def gather_results(plan, raw, group=None, device=None, selection=None):
+def gather_results(plan, raw, group=None, device=None, selection=None, marginal=None):
     """Every rank's GP records -> the assembled GPR dict of the whole sweep (SweepPlan.assemble) on every rank.
-    `selection`: this rank's tuned-sweep selection (RetrospectiveSweep.selection), gathered alongside."""
+    `selection`: this rank's tuned-sweep selection (RetrospectiveSweep.selection), `marginal`: this rank's
+    marginal-sweep records (RetrospectiveSweep.marginal), gathered alongside."""
     raw_all, meta, member = gather_records(plan, raw, group, device)
     sel_all = None if selection is None else gather_selection(selection, group, device)
-    return plan.assemble(raw_all, meta, member, selection=sel_all)
+    marg_all = None if marginal is None else gather_selection(marginal, group, device)
+    return plan.assemble(raw_all, meta, member, selection=sel_all, marginal=marg_all)
