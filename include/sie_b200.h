@@ -253,6 +253,34 @@ typedef struct SieGpMarginal {
 int sie_gp_grid_marginal(const SieGpResult* grid, int P, int n_grid, const double* q, int n_q,
                          SieGpResult* out, SieGpMarginal* stats, double* quant, void* stream);
 
+/* Ensemble pool per problem: the forecasts of M input-perturbed ensemble members pooled into one predictive
+ * distribution, each contributing member with weight 1 / M'.  rec [E][M][n_grid]: E ensemble problems (config, region,
+ * year) x M member slots x n_grid records per member -- n_grid = 1 for the forecast records of plain or tuned sweeps,
+ * n_grid = n_ell * n_sig for the grid records of marginalised sweeps.  Per member m, sie_gp_grid_marginal's
+ * arithmetic (A_m, e_k = exp(min - nlml_k), S0_m; same lane order): its mean mu_m = sum e mu / S0_m and variance
+ * v_m = sum e (v + (mu - mu_m)^2) / S0_m have the bits of that member's marginal record.  A member with A_m empty does
+ * not contribute; M' = the members that do.
+ *   out[e] = {fmean = sum mu_m / M', var_within = sum v_m / M', var_between = sum (mu_m - fmean)^2 / M' (second pass),
+ *             fvar = var_within + var_between, n_members = M'}
+ *   quant [E][n_q]: quantiles of F(x) = (1/M') sum_m (1/S0_m) sum_k e_mk Phi((x - mu_mk) / sd_mk) at the levels q
+ *          (0 < q < 1; v <= 0 is a point mass), by sie_gp_grid_marginal's bisection rule over the components with e > 0
+ * M' = 0: fmean, fvar, both variance terms and the quantiles NaN, n_members 0.  n_q == 0: q and quant may be NULL.
+ * scratch: at least sie_gp_ensemble_scratch_bytes(E, M, n_grid) bytes (the weighted components of every problem,
+ * 24 B per record).  Limits: M <= 1024 and M * n_grid < 2^31, else SIE_ERR_UNSUPPORTED.  One CTA per problem,
+ * sums in an order fixed by (M, n_grid): bit-reproducible, whichever launch filled which member slot.  Enqueue only. */
+typedef struct SieGpEnsemble {
+  double fmean;          /* mean of the pooled predictive distribution */
+  double fvar;           /* var_within + var_between */
+  double var_within;     /* mean over the contributing members of their predictive variance */
+  double var_between;    /* mean over the contributing members of (member mean - fmean)^2 */
+  int32_t n_members;     /* M' = members with at least one admissible record */
+  int32_t pad_;
+} SieGpEnsemble;         /* 40 bytes */
+
+int sie_gp_ensemble(const SieGpResult* rec, int E, int M, int n_grid, const double* q, int n_q,
+                    SieGpEnsemble* out, double* quant, void* scratch, size_t scratch_bytes, void* stream);
+size_t sie_gp_ensemble_scratch_bytes(int E, int M, int n_grid);
+
 /* ---------------------------------------------------------------------------------------------
  * Ingest (SURVEY.md 8(f) rows 1 and 4: the steps immediately before the hot path).
  * Replaces: readNSIDC                                          north/September1st.py:72-139

@@ -35,6 +35,11 @@ class SieGpMarginal(C.Structure):
     _fields_ = [("ess", C.c_double), ("w_max", C.c_double), ("n_admissible", c_i32), ("argmax", c_i32)]
 
 
+class SieGpEnsemble(C.Structure):
+    _fields_ = [("fmean", C.c_double), ("fvar", C.c_double), ("var_within", C.c_double), ("var_between", C.c_double),
+                ("n_members", c_i32), ("pad_", c_i32)]
+
+
 _SIGS = {
     "sie_abi_version": (C.c_int, []),
     "sie_last_error": (C.c_char_p, []),
@@ -62,6 +67,8 @@ _SIGS = {
                                     C.c_int, C.c_int, c_p, c_p, c_sz, c_p]),
     "sie_gp_grid_select": (C.c_int, [c_p, c_p, C.c_int, c_p, C.c_int, c_p, C.c_int, c_p, c_p, c_p]),
     "sie_gp_grid_marginal": (C.c_int, [c_p, C.c_int, C.c_int, c_p, C.c_int, c_p, c_p, c_p, c_p]),
+    "sie_gp_ensemble": (C.c_int, [c_p, C.c_int, C.c_int, C.c_int, c_p, C.c_int, c_p, c_p, c_p, c_sz, c_p]),
+    "sie_gp_ensemble_scratch_bytes": (c_sz, [C.c_int, C.c_int, C.c_int]),
     "sie_debug_gp_phases": (C.c_int, [C.POINTER(C.c_ulonglong)]),       # profiling aid (tools/gp_phases.py)
 }
 

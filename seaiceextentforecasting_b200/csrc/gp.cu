@@ -1222,6 +1222,259 @@ k_gp_grid_marginal(const SieGpResult* __restrict__ grid, int P, int n, const dou
   }
 }
 
+// Ensemble pool per problem (sie_gp_ensemble).  One CTA per ensemble problem e, whose records are [M][n]:
+//   1. one warp per member (members wp, wp + ENS_WARPS, ...): k_gp_grid_marginal's first two passes with the same
+//      helpers, lane striding and xor trees, so the member mean / variance have the bits of that member's marginal
+//      record; plus the member's count of e > 0 components and its part of the bracket [lo, hi]
+//   2. pooled moments over the contributing members (M' of them, weight 1 / M'), second pass for var_between
+//   3. the e > 0 components (w = e / S0_m, mu, sd) compacted into the CTA's slab of the scratch in (member, grid index)
+//      order, each member at the exclusive prefix sum of the counts
+//   4. bisection on F(x) = sum w Phi((x - mu) / sd) / M' for up to ENS_QB levels at once: one pass over the slab
+//      evaluates F at every active level's midpoint, so the slab is read once per halving, not once per level
+// Every sum runs over an index order fixed by (M, n) (per-thread strided sums, xor trees, then the warp sums added in
+// warp order), so the result does not depend on the schedule or on which batch filled which member slot.
+constexpr int ENS_WARPS = 8;
+constexpr int ENS_THREADS = ENS_WARPS * 32;
+constexpr int ENS_MAX_MEMBERS = 1024;   // per-member stats in static shared memory: 36 KB
+constexpr int ENS_QB = 4;               // quantile levels bisected together
+
+// Fixed-order CTA sum of NV values per thread; every thread gets the totals.  red: [NV][ENS_WARPS] shared.
+template <int NV>
+__device__ __forceinline__ void ens_block_sum(double (&v)[NV], double (*red)[ENS_WARPS]) {
+  const int wp = threadIdx.x >> 5;
+#pragma unroll
+  for (int j = 0; j < NV; ++j) v[j] = warp_sum_xor(v[j]);
+  __syncthreads();                                     // the previous call's readers are done with red
+  if ((threadIdx.x & 31) == 0) {
+#pragma unroll
+    for (int j = 0; j < NV; ++j) red[j][wp] = v[j];
+  }
+  __syncthreads();
+#pragma unroll
+  for (int j = 0; j < NV; ++j) {
+    double s = red[j][0];
+    for (int w = 1; w < ENS_WARPS; ++w) s = __dadd_rn(s, red[j][w]);
+    v[j] = s;
+  }
+}
+
+// f[j] <- F(x[j]) * M' for the levels j with bit j of `act` set, over the n_c compacted components.
+__device__ __forceinline__ void ens_cdf(const double* w, const double* mu, const double* sd, int n_c,
+                                        const double (&x)[ENS_QB], unsigned act, double (&f)[ENS_QB],
+                                        double (*red)[ENS_WARPS]) {
+#pragma unroll
+  for (int j = 0; j < ENS_QB; ++j) f[j] = 0.0;
+  for (int i = threadIdx.x; i < n_c; i += ENS_THREADS) {
+    const double wi = w[i], mi = mu[i], si = sd[i];
+#pragma unroll
+    for (int j = 0; j < ENS_QB; ++j)
+      if (act & (1u << j)) f[j] = __fma_rn(wi, si > 0.0 ? normcdf((x[j] - mi) / si) : (x[j] >= mi ? 1.0 : 0.0), f[j]);
+  }
+  ens_block_sum<ENS_QB>(f, red);
+}
+
+__global__ void __launch_bounds__(ENS_THREADS, 2)
+k_gp_ensemble(const SieGpResult* __restrict__ rec, int M, int n, const double* __restrict__ q, int n_q,
+              SieGpEnsemble* __restrict__ out, double* __restrict__ quant, double* __restrict__ scratch) {
+  __shared__ double s_mu[ENS_MAX_MEMBERS], s_v[ENS_MAX_MEMBERS], s_m[ENS_MAX_MEMBERS], s_s0[ENS_MAX_MEMBERS];
+  __shared__ int s_off[ENS_MAX_MEMBERS + 1];          // e > 0 components per member, then their exclusive prefix sum
+  __shared__ double s_red[ENS_QB][ENS_WARPS];
+  const int wp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int e = blockIdx.x;
+  const size_t cap = (size_t)M * n;
+  const SieGpResult* base = rec + (size_t)e * cap;
+  double* sw = scratch + (size_t)e * 3 * cap;          // this CTA's slab: w [cap], mu [cap], sd [cap]
+  double* smu = sw + cap;
+  double* ssd = smu + cap;
+
+  double lo = __longlong_as_double(0x7ff0000000000000LL), hi = -lo;
+  for (int mm = wp; mm < M; mm += ENS_WARPS) {
+    const SieGpResult* g = base + (size_t)mm * n;
+    double m;
+    int bi;
+    gp_grid_argmin_warp(g, n, lane, m, bi);
+    if (bi == SEL_NONE) {                              // A_m empty: the member does not contribute
+      if (lane == 0) s_off[mm] = 0;
+      continue;
+    }
+    double s0 = 0.0, s1 = 0.0;
+    int cnt = 0;
+    for (int k = lane; k < n; k += 32) {
+      double ek, mu, sd;
+      marg_component(&g[k], m, ek, mu, sd);
+      if (ek > 0.0) {
+        s0 = __dadd_rn(s0, ek);
+        s1 = __fma_rn(ek, mu, s1);
+        lo = fmin(lo, mu - 40.0 * sd);
+        hi = fmax(hi, mu + 40.0 * sd);
+        ++cnt;
+      }
+    }
+    s0 = warp_sum_xor(s0);
+    s1 = warp_sum_xor(s1);
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, off);
+    const double fmean = s1 / s0;
+    double sv = 0.0;
+    for (int k = lane; k < n; k += 32) {
+      double v;
+      if (gp_grid_admissible(&g[k], v)) {
+        const double ek = exp(m - v);
+        if (ek > 0.0) {
+          const double d = __ldg(&g[k].fmean) - fmean;
+          sv = __fma_rn(ek, __fma_rn(d, d, __ldg(&g[k].fvar)), sv);
+        }
+      }
+    }
+    sv = warp_sum_xor(sv);
+    if (lane == 0) {
+      s_mu[mm] = fmean;
+      s_v[mm] = sv / s0;
+      s_m[mm] = m;
+      s_s0[mm] = s0;
+      s_off[mm] = cnt;                                 // >= 1: the minimum has e = 1
+    }
+  }
+#pragma unroll
+  for (int off = 16; off > 0; off >>= 1) {
+    lo = fmin(lo, __shfl_xor_sync(0xffffffffu, lo, off));
+    hi = fmax(hi, __shfl_xor_sync(0xffffffffu, hi, off));
+  }
+  __syncthreads();
+  if (wp == 0) {                                       // exclusive scan of the counts: lane L owns a contiguous chunk
+    const int chunk = (M + 31) / 32, m0 = min(M, lane * chunk), m1 = min(M, m0 + chunk);
+    int t = 0;
+    for (int mm = m0; mm < m1; ++mm) t += s_off[mm];
+    int incl = t;
+#pragma unroll
+    for (int off = 1; off < 32; off <<= 1) {
+      const int o = __shfl_up_sync(0xffffffffu, incl, off);
+      if (lane >= off) incl += o;
+    }
+    int run = incl - t;
+    for (int mm = m0; mm < m1; ++mm) {
+      const int c = s_off[mm];
+      s_off[mm] = run;
+      run += c;
+    }
+    if (lane == 31) s_off[M] = incl;
+  }
+  __syncthreads();
+  double mv[3] = {0.0, 0.0, 0.0};                     // sum of the member means, of their variances, M'
+  for (int mm = threadIdx.x; mm < M; mm += ENS_THREADS) {
+    if (s_off[mm + 1] > s_off[mm]) {
+      mv[0] = __dadd_rn(mv[0], s_mu[mm]);
+      mv[1] = __dadd_rn(mv[1], s_v[mm]);
+      mv[2] += 1.0;
+    }
+  }
+  ens_block_sum<3>(mv, s_red);
+  const double mp = mv[2];
+  const int n_members = (int)mp;
+  const size_t qo = (size_t)e * n_q;
+  if (n_members == 0) {
+    if (threadIdx.x == 0) {
+      SieGpEnsemble r;
+      r.fmean = r.fvar = r.var_within = r.var_between = sie_nan();
+      r.n_members = 0;
+      r.pad_ = 0;
+      out[e] = r;
+    }
+    for (int i = threadIdx.x; i < n_q; i += ENS_THREADS) quant[qo + i] = sie_nan();
+    return;
+  }
+  const double fmean = mv[0] / mp, vw = mv[1] / mp;
+  double vb[1] = {0.0};
+  for (int mm = threadIdx.x; mm < M; mm += ENS_THREADS) {
+    if (s_off[mm + 1] > s_off[mm]) {
+      const double d = s_mu[mm] - fmean;
+      vb[0] = __fma_rn(d, d, vb[0]);
+    }
+  }
+  ens_block_sum<1>(vb, s_red);
+  if (threadIdx.x == 0) {
+    SieGpEnsemble r;
+    r.fmean = fmean;
+    r.var_within = vw;
+    r.var_between = vb[0] / mp;
+    r.fvar = r.var_within + r.var_between;
+    r.n_members = n_members;
+    r.pad_ = 0;
+    out[e] = r;
+  }
+  if (n_q == 0) return;
+
+  // bracket over every contributing component (fmin / fmax are exact: any order gives the same bits)
+  __syncthreads();
+  if (lane == 0) { s_red[0][wp] = lo; s_red[1][wp] = hi; }
+  __syncthreads();
+  lo = s_red[0][0];
+  hi = s_red[1][0];
+  for (int w = 1; w < ENS_WARPS; ++w) { lo = fmin(lo, s_red[0][w]); hi = fmax(hi, s_red[1][w]); }
+
+  for (int mm = wp; mm < M; mm += ENS_WARPS) {         // compaction, in (member, grid index) order
+    int off = s_off[mm];
+    if (s_off[mm + 1] == off) continue;
+    const SieGpResult* g = base + (size_t)mm * n;
+    const double m = s_m[mm], s0 = s_s0[mm];
+    for (int k0 = 0; k0 < n; k0 += 32) {
+      const int k = k0 + lane;
+      double ek = 0.0, mu = 0.0, sd = 0.0;
+      if (k < n) marg_component(&g[k], m, ek, mu, sd);
+      const unsigned bal = __ballot_sync(0xffffffffu, ek > 0.0);
+      if (ek > 0.0) {
+        const int i = off + __popc(bal & ((1u << lane) - 1u));
+        sw[i] = ek / s0;
+        smu[i] = mu;
+        ssd[i] = sd;
+      }
+      off += __popc(bal);
+    }
+  }
+  __syncthreads();                                     // the slab is visible to the whole CTA
+  const int n_c = s_off[M];
+
+  double x[ENS_QB], f[ENS_QB];
+#pragma unroll
+  for (int j = 0; j < ENS_QB; ++j) x[j] = j == 0 ? lo : hi;
+  ens_cdf(sw, smu, ssd, n_c, x, 3u, f, s_red);
+  const double f_lo = f[0] / mp, f_hi = f[1] / mp;
+  for (int i0 = 0; i0 < n_q; i0 += ENS_QB) {
+    const int nb = min(ENS_QB, n_q - i0);
+    double a[ENS_QB], b[ENS_QB], t[ENS_QB];
+    unsigned act = 0u;
+#pragma unroll
+    for (int j = 0; j < ENS_QB; ++j) {
+      t[j] = j < nb ? q[i0 + j] : 0.0;
+      a[j] = lo;
+      b[j] = hi;
+      if (j >= nb) continue;
+      if (f_lo >= t[j]) b[j] = lo;                     // a point mass at the lower end already holds q
+      else if (f_hi >= t[j]) act |= 1u << j;           // invariant F(a) < q <= F(b)
+    }                                                  // else: sum w rounds below q; hi is the upper end
+    for (int it = 0; it < 128 && act; ++it) {
+#pragma unroll
+      for (int j = 0; j < ENS_QB; ++j) {
+        if (!(act & (1u << j))) continue;
+        x[j] = 0.5 * a[j] + 0.5 * b[j];
+        if (x[j] == a[j] || x[j] == b[j]) act &= ~(1u << j);
+      }
+      if (!act) break;
+      ens_cdf(sw, smu, ssd, n_c, x, act, f, s_red);
+#pragma unroll
+      for (int j = 0; j < ENS_QB; ++j) {
+        if (!(act & (1u << j))) continue;
+        if (f[j] / mp >= t[j]) b[j] = x[j]; else a[j] = x[j];
+      }
+    }
+    if (threadIdx.x == 0) {
+#pragma unroll
+      for (int j = 0; j < ENS_QB; ++j)
+        if (j < nb) quant[qo + i0 + j] = b[j];
+    }
+  }
+}
+
 __host__ size_t gp_per_cta_bytes(int max_pred) {
   size_t d = (size_t)9 * max_pred * max_pred + (size_t)3 * MAXN * max_pred + (size_t)3 * max_pred + (size_t)MAXN * LDS;
   size_t bytes = d * sizeof(double) + (size_t)max_pred * sizeof(int);
@@ -1321,6 +1574,31 @@ extern "C" int sie_gp_grid_marginal(const SieGpResult* grid, int P, int n_grid, 
   SIE_CHECK_ARG(n_q == 0 || (q && quant), "q and quant must not be null when n_q > 0");
   k_gp_grid_marginal<<<(P - 1) / MARG_WARPS + 1, MARG_WARPS * 32, 0, (cudaStream_t)stream>>>(
       grid, P, n_grid, q, n_q, out, stats, quant);
+  SIE_CHECK_LAUNCH();
+  return SIE_OK;
+}
+
+extern "C" size_t sie_gp_ensemble_scratch_bytes(int E, int M, int n_grid) {
+  if (E < 1 || M < 1 || n_grid < 1) return 0;
+  return (size_t)E * (size_t)M * (size_t)n_grid * 3 * sizeof(double);
+}
+
+extern "C" int sie_gp_ensemble(const SieGpResult* rec, int E, int M, int n_grid, const double* q, int n_q,
+                               SieGpEnsemble* out, double* quant, void* scratch, size_t scratch_bytes, void* stream) {
+  SIE_CHECK_ARG(rec && out && scratch, "null pointer");
+  SIE_CHECK_ARG(E > 0 && M > 0 && n_grid > 0, "E, M and n_grid must be positive");
+  SIE_CHECK_ARG(n_q >= 0, "n_q must not be negative");
+  SIE_CHECK_ARG(n_q == 0 || (q && quant), "q and quant must not be null when n_q > 0");
+  if (M > ENS_MAX_MEMBERS) {
+    sie_set_error("%s: M = %d members, at most %d are supported", __func__, M, ENS_MAX_MEMBERS);
+    return SIE_ERR_UNSUPPORTED;
+  }
+  if ((long long)M * n_grid >= (1LL << 31)) {
+    sie_set_error("%s: M * n_grid = %lld records per problem, must be below 2^31", __func__, (long long)M * n_grid);
+    return SIE_ERR_UNSUPPORTED;
+  }
+  SIE_CHECK_ARG(scratch_bytes >= sie_gp_ensemble_scratch_bytes(E, M, n_grid), "scratch too small");
+  k_gp_ensemble<<<E, ENS_THREADS, 0, (cudaStream_t)stream>>>(rec, M, n_grid, q, n_q, out, quant, (double*)scratch);
   SIE_CHECK_LAUNCH();
   return SIE_OK;
 }

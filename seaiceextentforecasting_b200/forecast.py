@@ -11,6 +11,7 @@ from __future__ import annotations
 import ctypes as C
 
 import os
+import weakref
 
 import numpy as np
 import torch
@@ -223,6 +224,52 @@ def grid_marginal(grid_dev, P, n_grid, q_dev, out_dev, stats_dev, quant_dev):
     rc = _lib.load().sie_gp_grid_marginal(_ptr(grid_dev), int(P), int(n_grid), _ptr(q_dev) if n_q else null, n_q,
                                           _ptr(out_dev), _ptr(stats_dev), _ptr(quant_dev) if n_q else null, _stream())
     _lib.check(rc, "sie_gp_grid_marginal")
+
+
+# SieGpEnsemble (include/sie_b200.h): one ensemble problem's pooled predictive distribution (sie_gp_ensemble)
+GP_ENSEMBLE_DTYPE = np.dtype([("fmean", "<f8"), ("fvar", "<f8"), ("var_within", "<f8"), ("var_between", "<f8"),
+                              ("n_members", "<i4"), ("pad_", "<i4")])
+assert GP_ENSEMBLE_DTYPE.itemsize == C.sizeof(_lib.SieGpEnsemble) == 40
+
+
+def ensemble_records(pooled, quant):
+    """pooled: GP_ENSEMBLE_DTYPE [E] (or its bytes), quant: float64 [E][n_q] -> GP_ENSEMBLE_DTYPE's fields plus
+    `quantiles` (float64 [n_q], detrended) per ensemble problem."""
+    pooled = np.asarray(pooled).view(GP_ENSEMBLE_DTYPE).reshape(-1)
+    quant = np.asarray(quant, dtype=np.float64).reshape(-1)
+    quant = quant.reshape(len(pooled), quant.size // max(1, len(pooled)))
+    rec = np.empty(len(pooled), dtype=np.dtype(GP_ENSEMBLE_DTYPE.descr + [("quantiles", "<f8", (quant.shape[1],))]))
+    for f in GP_ENSEMBLE_DTYPE.names:
+        rec[f] = pooled[f]
+    rec["quantiles"] = quant
+    return rec
+
+
+def gp_ensemble_scratch_bytes(E, M, n_grid):
+    return int(_lib.load().sie_gp_ensemble_scratch_bytes(int(E), int(M), int(n_grid)))
+
+
+def gp_ensemble(rec_dev, E, M, n_grid, q_dev, out_dev, quant_dev, scratch_dev):
+    """sie_gp_ensemble on the current stream: out_dev [E] (GP_ENSEMBLE_DTYPE) <- the pool of the M members' records
+    rec_dev [E][M][n_grid] of every ensemble problem, quant_dev [E][n_q] <- its quantiles at the levels q_dev [n_q]
+    (q_dev None: none).  scratch_dev: at least gp_ensemble_scratch_bytes(E, M, n_grid) bytes."""
+    n_q = 0 if q_dev is None else q_dev.numel()
+    null = C.c_void_p(0)
+    rc = _lib.load().sie_gp_ensemble(_ptr(rec_dev), int(E), int(M), int(n_grid), _ptr(q_dev) if n_q else null, n_q,
+                                     _ptr(out_dev), _ptr(quant_dev) if n_q else null, _ptr(scratch_dev),
+                                     scratch_dev.numel() * scratch_dev.element_size(), _stream())
+    _lib.check(rc, "sie_gp_ensemble")
+
+
+def ensemble_slots(plan, n_members):
+    """The ensemble problems of a single-rank SweepPlan and where its records go in an ensemble store
+    [E][n_members][n_grid]: (meta int64 [E][3] = the sorted (config index, region index, year) triples, rows int64 [P]
+    = e * n_members + member of every problem, in the plan's current problem order, partition_sst's included)."""
+    meta = np.array(sorted({tuple(int(v) for v in m) for m in plan.prob_meta}), dtype=np.int64).reshape(-1, 3)
+    e_of = {tuple(m): e for e, m in enumerate(meta.tolist())}
+    rows = np.array([e_of[tuple(int(v) for v in m)] * int(n_members) + int(mb)
+                     for m, mb in zip(plan.prob_meta, plan.prob_member)], dtype=np.int64)
+    return meta, rows
 
 
 class _SeriesSet:
@@ -492,7 +539,7 @@ class SweepPlan:
                     for mm in range(self.members)]
         return self._assemble_one(raw, meta, selection, marginal)
 
-    def _assemble_one(self, raw, meta, selection=None, marginal=None):
+    def _assemble_one(self, raw, meta, selection=None, marginal=None, ensemble=None):
         m = np.asarray(meta, dtype=np.int64).reshape(-1, 3)
         out = {}
         if m.shape[0] == 0:
@@ -522,6 +569,12 @@ class SweepPlan:
                     qs = marginal["quantiles"][sel]
                     items += [("_grid_index", marginal["argmax"][sel]), ("_ess", marginal["ess"][sel]),
                               ("_w_max", marginal["w_max"][sel]), ("_quantiles", qs),
+                              ("_quantiles_rt", qs + line_last[:, None])]
+                if ensemble is not None:
+                    qs = ensemble["quantiles"][sel]
+                    items += [("_var_within", ensemble["var_within"][sel]),
+                              ("_var_between", ensemble["var_between"][sel]),
+                              ("_n_members", ensemble["n_members"][sel]), ("_quantiles", qs),
                               ("_quantiles_rt", qs + line_last[:, None])]
                 for key, val in items:
                     arr = g.setdefault(reg + key, np.full((len(self.years),) + np.shape(val)[1:], np.nan))
@@ -1087,3 +1140,86 @@ class RetrospectiveSweep:
                 raise _lib.SieError(f"GP problems {bad.tolist()[:8]} selected more than max_pred = {self.gp.max_pred} "
                                     "predictors (or n + 1 > 64 samples): construct the sweep with a larger max_pred")
         return st
+
+
+class EnsembleForecast:
+    """The ensemble forecast of a perturbed-input ensemble: every member's predictive distribution of each (config,
+    region, year) pooled into one on the device (sie_gp_ensemble), each member with weight 1 / M' (M' = members with a
+    forecast there).  It carries the input uncertainty on top of the GP and hyper-parameter uncertainty that each
+    member's record holds: fvar = var_within (mean member variance) + var_between (spread of the member means).
+
+    sweep      : a single-rank RetrospectiveSweep; fixes the configs, years, SIE targets, hyper mode and grid every added
+                 sweep must share.  What is pooled per member: the forecast record of plain and tuned ("argmin")
+                 sweeps (n_grid = 1), all n_ell * n_sig grid records of marginalised sweeps (n_grid = the grid size;
+                 each member then enters as its grid marginal)
+    n_members  : member slots; every slot must be filled by add() before result()
+    quantiles  : levels in (0, 1) of the pooled distribution's quantiles
+
+    Device memory, allocated once here: the record store, 80 * E * n_members * n_grid bytes (E = configs x regions x
+    years; 14.2 GB for the 4-init north sweep at 1024 members x the 400-point grid), and the kernel's scratch,
+    24 * E * n_members * n_grid bytes (4.2 GB there).  The ensemble streams through one sweep batch by batch:
+    sweep.load_inputs(batch) -> upload() -> compute() -> add(sweep, first_member), then result()."""
+
+    def __init__(self, sweep, n_members, quantiles=DEFAULT_QUANTILES):
+        if sweep.plan.world > 1:
+            raise NotImplementedError("an ensemble forecast pools the members of a single-rank sweep (world = 1)")
+        self.n_members = int(n_members)
+        if self.n_members < 1:
+            raise ValueError(f"n_members must be positive, got {n_members}")
+        self.levels = check_levels(quantiles)
+        self.plan = sweep.plan
+        self._key = self._signature(sweep)
+        self.n_grid = len(sweep.tune.ells) * len(sweep.tune.sigs) if sweep.hyper_mode == "marginal" else 1
+        self.meta, _ = ensemble_slots(self.plan, self.n_members)
+        self.E = len(self.meta)
+        self._rb = self.n_grid * GP_RESULT_DTYPE.itemsize
+        self.store = torch.empty(self.E * self.n_members * self._rb, dtype=torch.uint8, device="cuda")
+        self._filled = np.zeros(self.E * self.n_members, dtype=bool)
+        self._rows = weakref.WeakKeyDictionary()          # sweep -> (host rows, device rows) of its problems
+        self._q_dev = h2d(self.levels) if self.levels.size else None
+        self._out = torch.empty(self.E * GP_ENSEMBLE_DTYPE.itemsize, dtype=torch.uint8, device="cuda")
+        self._quant = torch.empty(max(1, self.E * self.levels.size), dtype=torch.float64, device="cuda")
+        self._scratch = torch.empty(gp_ensemble_scratch_bytes(self.E, self.n_members, self.n_grid), dtype=torch.uint8,
+                                    device="cuda")
+        self.records = None                               # ensemble_records of the last result()
+
+    @staticmethod
+    def _signature(sweep):
+        p = sweep.plan
+        grid = None if sweep.tune is None else (sweep.tune.ells.tobytes(), sweep.tune.sigs.tobytes())
+        return (tuple(c.name for c in p.cfgs), tuple(p.years), tuple((k, v.tobytes()) for k, v in sorted(p.sie.items())),
+                sweep.hyper_mode, grid)
+
+    def add(self, sweep, first_member=0):
+        """Enqueue (current stream, no host sync) the copy of the records of `sweep`'s last compute() into member slots
+        first_member + 0 .. sweep.members - 1.  Raises ValueError for a sweep with other configs, years, SIE targets,
+        hyper mode or grid, or slots beyond n_members."""
+        if sweep.plan.world > 1:
+            raise NotImplementedError("an ensemble forecast pools the members of a single-rank sweep (world = 1)")
+        if self._signature(sweep) != self._key:
+            raise ValueError("the sweep's configs, years, SIE targets, hyper mode or grid differ from the ensemble's")
+        first = int(first_member)
+        if first < 0 or first + sweep.members > self.n_members:
+            raise ValueError(f"members {first}..{first + sweep.members - 1} do not fit the {self.n_members} slots")
+        rows = self._rows.get(sweep)
+        if rows is None:
+            host = ensemble_slots(sweep.plan, self.n_members)[1]
+            rows = self._rows[sweep] = (host, h2d(host))
+        host, dev = rows
+        src = sweep.tune.out if sweep.hyper_mode == "marginal" else sweep.gp.out
+        self.store.view(self.E * self.n_members, self._rb).index_copy_(
+            0, dev + first if first else dev, src[:sweep.P * self._rb].view(sweep.P, self._rb))
+        self._filled[host + first] = True
+
+    def result(self):
+        """Pool the store on the device and read it back (synchronises) -> the dict of a member's assembled forecast
+        ('<region>_fmean / _fvar / _fmean_rt' at 3 d.p., '_raw_*') for the ensemble forecast, plus '_var_within',
+        '_var_between', '_n_members', '_quantiles' and '_quantiles_rt' (re-trended like '_raw_fmean_rt').  NaN where no
+        member has a forecast.  SweepPlan.skill() reads it unchanged."""
+        if not self._filled.all():
+            miss = np.argwhere(~self._filled.reshape(self.E, self.n_members))
+            raise RuntimeError(f"{len(miss)} (problem, member) slots were never added, e.g. member {miss[0][1]}")
+        gp_ensemble(self.store, self.E, self.n_members, self.n_grid, self._q_dev, self._out, self._quant, self._scratch)
+        nq = self.levels.size
+        self.records = ensemble_records(self._out.cpu().numpy(), self._quant.cpu().numpy()[:self.E * nq])
+        return self.plan._assemble_one(self.records, self.meta, ensemble=self.records)
