@@ -1119,10 +1119,56 @@ __device__ __forceinline__ bool marg_component(const SieGpResult* __restrict__ r
   return true;
 }
 
+// Passes 1-2 of one grid's marginal (k_gp_grid_marginal, and every member of k_gp_ensemble, so that a member's mean and
+// variance have the bits of its marginal record): over the records g[0..n) whose admissible minimum is m, the
+// warp-reduced S0 = sum e, the mixture mean sum e mu / S0 and variance sum e (v + (mu - mean)^2) / S0 (second pass), |A|
+// and the number of e > 0 points.  Left per lane for the caller: s2 += e^2, and the bracket [lo, hi] of the e > 0
+// components (extended, not reset).  st not null: (e, mu, sd) of every point are staged in st[0..2][k].
+struct MargMoments {
+  double s0, fmean, fvar;
+  int n_admissible, n_positive;
+};
+__device__ __forceinline__ MargMoments marg_moments(const SieGpResult* __restrict__ g, int n, int lane, double m,
+                                                    double (*st)[MARG_STAGE], double& s2, double& lo, double& hi) {
+  double s0 = 0.0, s1 = 0.0;
+  int n_adm = 0, n_pos = 0;
+  for (int k = lane; k < n; k += 32) {
+    double e, mu, sd;
+    n_adm += marg_component(&g[k], m, e, mu, sd) ? 1 : 0;
+    if (st) { st[0][k] = e; st[1][k] = mu; st[2][k] = sd; }
+    if (e > 0.0) {
+      s0 = __dadd_rn(s0, e);
+      s2 = __fma_rn(e, e, s2);
+      s1 = __fma_rn(e, mu, s1);
+      lo = fmin(lo, mu - 40.0 * sd);
+      hi = fmax(hi, mu + 40.0 * sd);
+      ++n_pos;
+    }
+  }
+  s0 = warp_sum_xor(s0);
+  s1 = warp_sum_xor(s1);
+  n_adm = __reduce_add_sync(0xffffffffu, n_adm);       // integer sums: exact in any order
+  n_pos = __reduce_add_sync(0xffffffffu, n_pos);
+  const double fmean = s1 / s0;
+  double sv = 0.0;
+  for (int k = lane; k < n; k += 32) {
+    double v;
+    if (gp_grid_admissible(&g[k], v)) {
+      const double e = exp(m - v);
+      if (e > 0.0) {
+        const double d = __ldg(&g[k].fmean) - fmean;
+        sv = __fma_rn(e, __fma_rn(d, d, __ldg(&g[k].fvar)), sv);
+      }
+    }
+  }
+  sv = warp_sum_xor(sv);
+  return {s0, fmean, sv / s0, n_adm, n_pos};
+}
+
 __global__ void __launch_bounds__(MARG_WARPS * 32)
 k_gp_grid_marginal(const SieGpResult* __restrict__ grid, int P, int n, const double* __restrict__ q, int n_q,
                    SieGpResult* __restrict__ out, SieGpMarginal* __restrict__ stats, double* __restrict__ quant) {
-  __shared__ double s_e[MARG_WARPS][MARG_STAGE], s_mu[MARG_WARPS][MARG_STAGE], s_sd[MARG_WARPS][MARG_STAGE];
+  __shared__ double s_c[MARG_WARPS][3][MARG_STAGE];  // staged (e, mu, sd) of each warp's problem
   const int wp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int p = blockIdx.x * MARG_WARPS + wp;
   if (p >= P) return;                                  // whole warp: p is uniform across it
@@ -1144,43 +1190,16 @@ k_gp_grid_marginal(const SieGpResult* __restrict__ grid, int P, int n, const dou
     for (int i = lane; i < n_q; i += 32) quant[(size_t)p * n_q + i] = sie_nan();
     return;
   }
-  const bool staged = n <= MARG_STAGE;
-  double s0 = 0.0, s2 = 0.0, s1 = 0.0, lo = __longlong_as_double(0x7ff0000000000000LL), hi = -lo;
-  int cnt = 0;
-  for (int k = lane; k < n; k += 32) {
-    double e, mu, sd;
-    cnt += marg_component(&g[k], m, e, mu, sd) ? 1 : 0;
-    if (staged) { s_e[wp][k] = e; s_mu[wp][k] = mu; s_sd[wp][k] = sd; }
-    if (e > 0.0) {
-      s0 = __dadd_rn(s0, e);
-      s2 = __fma_rn(e, e, s2);
-      s1 = __fma_rn(e, mu, s1);
-      lo = fmin(lo, mu - 40.0 * sd);
-      hi = fmax(hi, mu + 40.0 * sd);
-    }
-  }
-  s0 = warp_sum_xor(s0);
+  double (*st)[MARG_STAGE] = n <= MARG_STAGE ? s_c[wp] : nullptr;
+  double s2 = 0.0, lo = __longlong_as_double(0x7ff0000000000000LL), hi = -lo;
+  const MargMoments mo = marg_moments(g, n, lane, m, st, s2, lo, hi);
+  const double s0 = mo.s0;
   s2 = warp_sum_xor(s2);
-  s1 = warp_sum_xor(s1);
 #pragma unroll
   for (int off = 16; off > 0; off >>= 1) {
-    cnt += __shfl_xor_sync(0xffffffffu, cnt, off);
     lo = fmin(lo, __shfl_xor_sync(0xffffffffu, lo, off));
     hi = fmax(hi, __shfl_xor_sync(0xffffffffu, hi, off));
   }
-  const double fmean = s1 / s0;
-  double sv = 0.0;
-  for (int k = lane; k < n; k += 32) {
-    double v;
-    if (gp_grid_admissible(&g[k], v)) {
-      const double e = exp(m - v);
-      if (e > 0.0) {
-        const double d = __ldg(&g[k].fmean) - fmean;
-        sv = __fma_rn(e, __fma_rn(d, d, __ldg(&g[k].fvar)), sv);
-      }
-    }
-  }
-  sv = warp_sum_xor(sv);
   __syncwarp();                                        // the staged components are visible to the whole warp
 
   // F(x) = sum_k e_k Phi((x - mu_k) / sd_k) / S0, a point mass (sd = 0) counting from x = mu on (right-continuous)
@@ -1188,7 +1207,7 @@ k_gp_grid_marginal(const SieGpResult* __restrict__ grid, int P, int n, const dou
     double f = 0.0;
     for (int k = lane; k < n; k += 32) {
       double e, mu, sd;
-      if (staged) { e = s_e[wp][k]; mu = s_mu[wp][k]; sd = s_sd[wp][k]; }
+      if (st) { e = st[0][k]; mu = st[1][k]; sd = st[2][k]; }
       else marg_component(&g[k], m, e, mu, sd);
       if (e > 0.0) f = __fma_rn(e, sd > 0.0 ? normcdf((x - mu) / sd) : (x >= mu ? 1.0 : 0.0), f);
     }
@@ -1209,23 +1228,23 @@ k_gp_grid_marginal(const SieGpResult* __restrict__ grid, int P, int n, const dou
   }
   if (lane == 0) {
     SieGpResult r = g[bi];
-    r.fmean = fmean;
-    r.fvar = sv / s0;
-    r.nlml = m - log(s0) + log((double)cnt);
+    r.fmean = mo.fmean;
+    r.fvar = mo.fvar;
+    r.nlml = m - log(s0) + log((double)mo.n_admissible);
     out[p] = r;
     SieGpMarginal s;
     s.ess = s0 * s0 / s2;
     s.w_max = 1.0 / s0;
-    s.n_admissible = cnt;
+    s.n_admissible = mo.n_admissible;
     s.argmax = bi;
     stats[p] = s;
   }
 }
 
 // Ensemble pool per problem (sie_gp_ensemble).  One CTA per ensemble problem e, whose records are [M][n]:
-//   1. one warp per member (members wp, wp + ENS_WARPS, ...): k_gp_grid_marginal's first two passes with the same
-//      helpers, lane striding and xor trees, so the member mean / variance have the bits of that member's marginal
-//      record; plus the member's count of e > 0 components and its part of the bracket [lo, hi]
+//   1. one warp per member (members wp, wp + ENS_WARPS, ...): k_gp_grid_marginal's first two passes (marg_moments), so
+//      the member mean / variance have the bits of that member's marginal record; plus the member's count of e > 0
+//      components and its part of the bracket [lo, hi]
 //   2. pooled moments over the contributing members (M' of them, weight 1 / M'), second pass for var_between
 //   3. the e > 0 components (w = e / S0_m, mu, sd) compacted into the CTA's slab of the scratch in (member, grid index)
 //      order, each member at the exclusive prefix sum of the counts
@@ -1297,42 +1316,14 @@ k_gp_ensemble(const SieGpResult* __restrict__ rec, int M, int n, const double* _
       if (lane == 0) s_off[mm] = 0;
       continue;
     }
-    double s0 = 0.0, s1 = 0.0;
-    int cnt = 0;
-    for (int k = lane; k < n; k += 32) {
-      double ek, mu, sd;
-      marg_component(&g[k], m, ek, mu, sd);
-      if (ek > 0.0) {
-        s0 = __dadd_rn(s0, ek);
-        s1 = __fma_rn(ek, mu, s1);
-        lo = fmin(lo, mu - 40.0 * sd);
-        hi = fmax(hi, mu + 40.0 * sd);
-        ++cnt;
-      }
-    }
-    s0 = warp_sum_xor(s0);
-    s1 = warp_sum_xor(s1);
-#pragma unroll
-    for (int off = 16; off > 0; off >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, off);
-    const double fmean = s1 / s0;
-    double sv = 0.0;
-    for (int k = lane; k < n; k += 32) {
-      double v;
-      if (gp_grid_admissible(&g[k], v)) {
-        const double ek = exp(m - v);
-        if (ek > 0.0) {
-          const double d = __ldg(&g[k].fmean) - fmean;
-          sv = __fma_rn(ek, __fma_rn(d, d, __ldg(&g[k].fvar)), sv);
-        }
-      }
-    }
-    sv = warp_sum_xor(sv);
+    double s2 = 0.0;
+    const MargMoments mo = marg_moments(g, n, lane, m, nullptr, s2, lo, hi);
     if (lane == 0) {
-      s_mu[mm] = fmean;
-      s_v[mm] = sv / s0;
+      s_mu[mm] = mo.fmean;
+      s_v[mm] = mo.fvar;
       s_m[mm] = m;
-      s_s0[mm] = s0;
-      s_off[mm] = cnt;                                 // >= 1: the minimum has e = 1
+      s_s0[mm] = mo.s0;
+      s_off[mm] = mo.n_positive;                       // >= 1: the minimum has e = 1
     }
   }
 #pragma unroll

@@ -94,6 +94,15 @@ def skill(obs_rt, forecast_rt, obs_dt, forecast_dt):
 # ------------------------------------------------------------------------------------------------
 # batched GP
 # ------------------------------------------------------------------------------------------------
+def _series_args(sic, sst):
+    """(anomaly, n_areas, MA, Tstride) of the SIC node series, then of the SST ones (null / 0 without SST): the series
+    arguments of sie_gp_forecast and sie_gp_hyper_grid."""
+    if sst is None:
+        return _ptr(sic.anomaly), _ptr(sic.n_areas), sic.MA, sic.Tstride, C.c_void_p(0), C.c_void_p(0), 0, 0
+    return (_ptr(sic.anomaly), _ptr(sic.n_areas), sic.MA, sic.Tstride,
+            _ptr(sst.anomaly), _ptr(sst.n_areas), sst.MA, sst.Tstride)
+
+
 class GpBatch:
     """P GP problems over one or two anomaly sets held by NetworkBatch objects."""
 
@@ -114,23 +123,17 @@ class GpBatch:
         out = self.out if out is None else out
         isz = GP_PROBLEM_DTYPE.itemsize
         osz = GP_RESULT_DTYPE.itemsize
-        rc = self.lib.sie_gp_forecast(
-            _ptr(prob_dev[p0 * isz:]), p1 - p0, _ptr(y_dev), _ptr(sic.anomaly), _ptr(sic.n_areas), sic.MA, sic.Tstride,
-            _ptr(sst.anomaly) if sst is not None else C.c_void_p(0),
-            _ptr(sst.n_areas) if sst is not None else C.c_void_p(0),
-            sst.MA if sst is not None else 0, sst.Tstride if sst is not None else 0,
-            self.max_pred, _ptr(out[p0 * osz:]), _ptr(self.scratch), self.scratch_bytes, _stream())
+        rc = self.lib.sie_gp_forecast(_ptr(prob_dev[p0 * isz:]), p1 - p0, _ptr(y_dev), *_series_args(sic, sst),
+                                      self.max_pred, _ptr(out[p0 * osz:]), _ptr(self.scratch), self.scratch_bytes,
+                                      _stream())
         _lib.check(rc, "sie_gp_forecast")
 
     def run_grid(self, prob_dev, sig_grid_dev, n_sig, y_dev, sic, sst, out):
         """Hyper-parameter grid: problem p fixes l = prob[p].ell; every sig_grid[k] is evaluated from the same
         expm / X Sigma X^T (sie_gp_hyper_grid).  `out`: uint8 device buffer of P * n_sig result records."""
-        rc = self.lib.sie_gp_hyper_grid(
-            _ptr(prob_dev), self.P, _ptr(sig_grid_dev), int(n_sig), _ptr(y_dev), _ptr(sic.anomaly), _ptr(sic.n_areas),
-            sic.MA, sic.Tstride, _ptr(sst.anomaly) if sst is not None else C.c_void_p(0),
-            _ptr(sst.n_areas) if sst is not None else C.c_void_p(0), sst.MA if sst is not None else 0,
-            sst.Tstride if sst is not None else 0, self.max_pred, _ptr(out), _ptr(self.scratch), self.scratch_bytes,
-            _stream())
+        rc = self.lib.sie_gp_hyper_grid(_ptr(prob_dev), self.P, _ptr(sig_grid_dev), int(n_sig), _ptr(y_dev),
+                                        *_series_args(sic, sst), self.max_pred, _ptr(out), _ptr(self.scratch),
+                                        self.scratch_bytes, _stream())
         _lib.check(rc, "sie_gp_hyper_grid")
 
     def results(self):
@@ -189,6 +192,18 @@ assert GP_MARGINAL_DTYPE.itemsize == C.sizeof(_lib.SieGpMarginal)
 DEFAULT_QUANTILES = (0.05, 0.5, 0.95)
 
 
+def _with_quantiles(recs, dtype, quant):
+    """recs: `dtype` [N] (or its bytes), quant: float64 [N][n_q] -> `dtype`'s fields plus `quantiles` [N]."""
+    recs = np.asarray(recs).view(dtype).reshape(-1)
+    quant = np.asarray(quant, dtype=np.float64).reshape(-1)
+    quant = quant.reshape(len(recs), quant.size // max(1, len(recs)))
+    rec = np.empty(len(recs), dtype=np.dtype(dtype.descr + [("quantiles", "<f8", (quant.shape[1],))]))
+    for f in dtype.names:
+        rec[f] = recs[f]
+    rec["quantiles"] = quant
+    return rec
+
+
 def marginal_dtype(n_q):
     """Per-problem record of a marginalised forecast: GP_MARGINAL_DTYPE's fields plus `quantiles`, a float64 sub-array
     of the n_q predictive quantiles (detrended).  Its length is the number of levels, hence a function of n_q."""
@@ -197,14 +212,7 @@ def marginal_dtype(n_q):
 
 def marginal_records(stats, quant):
     """stats: GP_MARGINAL_DTYPE [P] (or its bytes), quant: float64 [P][n_q] -> marginal_dtype(n_q) [P]."""
-    stats = np.asarray(stats).view(GP_MARGINAL_DTYPE).reshape(-1)
-    quant = np.asarray(quant, dtype=np.float64).reshape(-1)
-    quant = quant.reshape(len(stats), quant.size // max(1, len(stats)))
-    rec = np.empty(len(stats), dtype=marginal_dtype(quant.shape[1]))
-    for f in GP_MARGINAL_DTYPE.names:
-        rec[f] = stats[f]
-    rec["quantiles"] = quant
-    return rec
+    return _with_quantiles(stats, GP_MARGINAL_DTYPE, quant)
 
 
 def check_levels(quantiles):
@@ -235,14 +243,7 @@ assert GP_ENSEMBLE_DTYPE.itemsize == C.sizeof(_lib.SieGpEnsemble) == 40
 def ensemble_records(pooled, quant):
     """pooled: GP_ENSEMBLE_DTYPE [E] (or its bytes), quant: float64 [E][n_q] -> GP_ENSEMBLE_DTYPE's fields plus
     `quantiles` (float64 [n_q], detrended) per ensemble problem."""
-    pooled = np.asarray(pooled).view(GP_ENSEMBLE_DTYPE).reshape(-1)
-    quant = np.asarray(quant, dtype=np.float64).reshape(-1)
-    quant = quant.reshape(len(pooled), quant.size // max(1, len(pooled)))
-    rec = np.empty(len(pooled), dtype=np.dtype(GP_ENSEMBLE_DTYPE.descr + [("quantiles", "<f8", (quant.shape[1],))]))
-    for f in GP_ENSEMBLE_DTYPE.names:
-        rec[f] = pooled[f]
-    rec["quantiles"] = quant
-    return rec
+    return _with_quantiles(pooled, GP_ENSEMBLE_DTYPE, quant)
 
 
 def gp_ensemble_scratch_bytes(E, M, n_grid):
@@ -287,51 +288,50 @@ class _SeriesSet:
         self.Tstride = n + 1
 
 
-def _one_problem(n, anoms_sst, rule, alpha, zscore, want_grad):
-    prob = np.zeros(1, dtype=GP_PROBLEM_DTYPE)
-    prob["job_sic"] = 0
-    prob["job_sst"] = 0 if anoms_sst is not None else -1
-    prob["n"] = n
-    prob["rule"] = rule
-    prob["zscore"] = int(zscore)
-    prob["want_grad"] = int(want_grad)
-    prob["r_sel"] = r_crit_pearson(n, alpha) if rule == RULE_POS_SIG else 0.0
-    return prob
+class _OneProblem:
+    """One forecast problem from node series given as dicts (the reference's `dataset['anoms']`) on the device: its
+    targets `y`, node series `s1` (SIC) and `s2` (SST, None without), host problem record `prob` [1] (l, sigma_n~ left
+    0) and `gp`, a GpBatch of P problems sized for its predictors."""
+
+    def __init__(self, y, anoms_sic, anoms_sst, rule, alpha, zscore, want_grad, P=1):
+        require_cuda()
+        y = np.asarray(y, dtype=np.float64).reshape(-1)
+        n = y.size
+        self.y = h2d(y)
+        self.s1 = _SeriesSet(anoms_sic, n)
+        self.s2 = _SeriesSet(anoms_sst, n) if anoms_sst is not None else None
+        self.prob = np.zeros(1, dtype=GP_PROBLEM_DTYPE)
+        self.prob["job_sic"] = 0
+        self.prob["job_sst"] = 0 if anoms_sst is not None else -1
+        self.prob["n"] = n
+        self.prob["rule"] = rule
+        self.prob["zscore"] = int(zscore)
+        self.prob["want_grad"] = int(want_grad)
+        self.prob["r_sel"] = r_crit_pearson(n, alpha) if rule == RULE_POS_SIG else 0.0
+        npred = self.s1.MA + (self.s2.MA if self.s2 is not None else 0)
+        self.gp = GpBatch(P, max_pred=max(4, npred))
 
 
 def forecast(y, anoms_sic, anoms_sst=None, rule=0, alpha=0.05, zscore=False, ell=1.0, sig=1.0, want_grad=False):
     """One GP forecast from node series given as dicts (the reference's `dataset['anoms']`), i.e. the body of
     `forecast()` for one region (north/June1st.py:214-277).  Returns the raw result record."""
-    require_cuda()
-    y = np.asarray(y, dtype=np.float64).reshape(-1)
-    n = y.size
-    s1 = _SeriesSet(anoms_sic, n)
-    s2 = _SeriesSet(anoms_sst, n) if anoms_sst is not None else None
-    prob = _one_problem(n, anoms_sst, rule, alpha, zscore, want_grad)
-    prob["ell"] = ell
-    prob["sig"] = sig
-    npred = s1.MA + (s2.MA if s2 is not None else 0)
-    gp = GpBatch(1, max_pred=max(4, npred))
-    gp.run(h2d(prob.view(np.uint8)), h2d(y), s1, s2)
-    return gp.results()[0]
+    one = _OneProblem(y, anoms_sic, anoms_sst, rule, alpha, zscore, want_grad)
+    one.prob["ell"] = ell
+    one.prob["sig"] = sig
+    one.gp.run(h2d(one.prob.view(np.uint8)), one.y, one.s1, one.s2)
+    return one.gp.results()[0]
 
 
 def _grid_on_device(y, anoms_sic, anoms_sst, rule, alpha, zscore, ells, sigs, want_grad):
     """One problem's (l, sigma_n~) grid records, left on the device: (uint8 buffer of [len(ells)][len(sigs)] records,
     ells, sigs); ells / sigs None are the reference's grids."""
-    require_cuda()
     ells = np.logspace(-7, 2, 20) if ells is None else np.asarray(ells, dtype=np.float64)
     sigs = np.logspace(-3, 9, 20) if sigs is None else np.asarray(sigs, dtype=np.float64)
-    y = np.asarray(y, dtype=np.float64).reshape(-1)
-    n = y.size
-    s1 = _SeriesSet(anoms_sic, n)
-    s2 = _SeriesSet(anoms_sst, n) if anoms_sst is not None else None
-    prob = np.repeat(_one_problem(n, anoms_sst, rule, alpha, zscore, want_grad), len(ells))
+    one = _OneProblem(y, anoms_sic, anoms_sst, rule, alpha, zscore, want_grad, P=len(ells))
+    prob = np.repeat(one.prob, len(ells))
     prob["ell"] = ells
-    npred = s1.MA + (s2.MA if s2 is not None else 0)
-    gp = GpBatch(len(ells), max_pred=max(4, npred))
     out = torch.empty(len(ells) * len(sigs) * GP_RESULT_DTYPE.itemsize, dtype=torch.uint8, device="cuda")
-    gp.run_grid(h2d(prob.view(np.uint8)), h2d(sigs), len(sigs), h2d(y), s1, s2, out)
+    one.gp.run_grid(h2d(prob.view(np.uint8)), h2d(sigs), len(sigs), one.y, one.s1, one.s2, out)
     return out, ells, sigs
 
 
@@ -379,23 +379,16 @@ class MliiObjective:
     uploaded once, every call evaluates the negative log marginal likelihood and its gradient on the device."""
 
     def __init__(self, y, anoms_sic, anoms_sst=None, rule=0, alpha=0.05, zscore=False):
-        require_cuda()
-        y = np.asarray(y, dtype=np.float64).reshape(-1)
-        n = y.size
-        self.s1 = _SeriesSet(anoms_sic, n)
-        self.s2 = _SeriesSet(anoms_sst, n) if anoms_sst is not None else None
-        self.prob = _one_problem(n, anoms_sst, rule, alpha, zscore, True)
-        self.y = h2d(y)
-        npred = self.s1.MA + (self.s2.MA if self.s2 is not None else 0)
-        self.gp = GpBatch(1, max_pred=max(4, npred))
+        self.one = _OneProblem(y, anoms_sic, anoms_sst, rule, alpha, zscore, True)
         self.evaluations = 0
 
     def record(self, theta):
-        self.prob["ell"] = float(np.exp(theta[0]))
-        self.prob["sig"] = float(np.exp(theta[1]))
-        self.gp.run(h2d(self.prob.view(np.uint8)), self.y, self.s1, self.s2)
+        one = self.one
+        one.prob["ell"] = float(np.exp(theta[0]))
+        one.prob["sig"] = float(np.exp(theta[1]))
+        one.gp.run(h2d(one.prob.view(np.uint8)), one.y, one.s1, one.s2)
         self.evaluations += 1
-        return self.gp.results()[0]
+        return one.gp.results()[0]
 
     def __call__(self, theta):
         r = self.record(theta)
@@ -596,6 +589,11 @@ class SweepPlan:
         return out
 
 
+def _members(x, n):
+    """One member's input or a list (tuple) of them -> a list; a single input stands for all n members."""
+    return list(x) if isinstance(x, (list, tuple)) else [x] * n
+
+
 class RetrospectiveSweep:
     """years fmin..fmax x the given init-month configs x 3 regions, in one device-resident batch.
 
@@ -630,15 +628,13 @@ class RetrospectiveSweep:
         if levels.size and hyper_mode != "marginal":
             raise ValueError("quantiles are computed by marginal sweeps only (hyper_mode='marginal')")
         require_cuda()
-        member_fields = list(sic_fields) if isinstance(sic_fields, (list, tuple)) else [sic_fields]
+        member_fields = _members(sic_fields, 1)
         self.members = len(member_fields)
         self.plan = plan = SweepPlan(config_names, sie, fmin, fmax, significance, rank, world, members=self.members)
         self.cfgs, self.years, self.fmin, self.fmax = plan.cfgs, plan.years, plan.fmin, plan.fmax
-        first = np.asarray(member_fields[0][self.cfgs[0].name])
-        self.X, self.Y, self.Tfull = first.shape
+        self.X, self.Y, self.Tfull = np.shape(member_fields[0][self.cfgs[0].name])
         assert self.Tfull >= self.fmax - FIRST_YEAR + 1
-        self.sic_host = np.stack([np.ascontiguousarray(mf[c.name], dtype=np.float64).reshape(
-            self.X * self.Y, self.Tfull) for mf in member_fields for c in self.cfgs])      # [member * n_configs + ci]
+        self.sic_host = self._stack_sic(member_fields)      # [member * n_configs + ci]
         self.psar_host = np.sqrt(np.asarray(psar, dtype=np.float64)).reshape(-1)     # ComplexNetworks.py:298-299
         self.use_sst = plan.use_sst and len(plan.sst_years) > 0
         # node capacity: a cell is a node of window T when its first T samples are NaN-free (detrend() fits the prefix),
@@ -652,11 +648,8 @@ class RetrospectiveSweep:
                                 max_areas=max_areas, keep_R=keep_R)
         self.sst = None
         if self.use_sst:
-            sst_members = list(sst_field) if isinstance(sst_field, (list, tuple)) else [sst_field] * self.members
-            assert len(sst_members) == self.members
-            s = np.stack([np.ascontiguousarray(f, dtype=np.float64) for f in sst_members])
-            self.Xs, self.Ys = s.shape[1], s.shape[2]
-            self.sst_host = s.reshape(self.members, self.Xs * self.Ys, self.Tfull)
+            self.Xs, self.Ys = np.shape(_members(sst_field, 1)[0])[:2]
+            self.sst_host = self._stack_sst(sst_field)
             self.lat_host = np.sqrt(np.cos(np.radians(np.asarray(sst_lat, dtype=np.float64)))).reshape(-1)  # :296-297
             Tmin_s = int(plan.sst_T.min())
             n_up = int(max((~np.isnan(f[:, :Tmin_s]).any(axis=1)).sum() for f in self.sst_host))
@@ -700,7 +693,6 @@ class RetrospectiveSweep:
             for (jr, sr, pr) in self.waves:
                 ok = ok and bool((plan.prob["job_sic"][pr[0]:pr[1]] >= jr[0]).all())
         self.multi_wave = bool(ok and len(self.waves) > 1)
-        self.two_waves = self.multi_wave       # (name kept for callers)
         self.gp_wave = [GpBatch(max(1, pr[1] - pr[0]), max_pred=max_pred) for (_, _, pr) in self.waves[1:]] \
             if self.multi_wave else []
         # Within a wave the problems that read no SST network come first: they only wait for the wave's SIC networks,
@@ -715,10 +707,11 @@ class RetrospectiveSweep:
         self._streams = None
         self._graph = None
         self.use_graph = bool(os.environ.get("SIE_GRAPH"))      # opt-in: see compute()
-        self.dev = None
         # pinned staging buffers so every step pays a real host->device copy
         self._pin = {name: torch.from_numpy(np.ascontiguousarray(arr)).pin_memory()
                      for name, arr in self._host_inputs().items()}
+        self.dev = self._device_inputs()
+        self._dev2, self._copy_stream = None, None     # run_many's second input set and its copy stream
         self._h2d_done = None                  # event after the last enqueued copy out of self._pin (load_inputs)
         self._grids = {}                       # (ells, sigs) -> _GridBuffers (hyper_grid() and the tuned step)
         self.tune = None
@@ -739,6 +732,43 @@ class RetrospectiveSweep:
                 self._mstats = torch.empty(self.P * GP_MARGINAL_DTYPE.itemsize, dtype=torch.uint8, device="cuda")
                 self._quant = torch.empty(max(1, self.P * levels.size), dtype=torch.float64, device="cuda")
             self._gp_tuned = {}                # GP launch range -> GpBatch of its grid (its scratch also serves the forecast)
+        # what a step reads back, each sliced to the bytes read (decoded by _decode); pinned host copies per slot:
+        # 0 / 1 for run_many's two steps in flight, 2 for download()
+        self._d2h = [self.gp.out[:self.P * GP_RESULT_DTYPE.itemsize]]
+        if self.hyper_mode == "argmin":
+            self._d2h += [self._tuned, self._best]
+        elif self.hyper_mode == "marginal":
+            self._d2h += [self._mstats, self._quant[:self.P * levels.size]]
+        self._pinned = [None] * 3
+
+    def _stack_sic(self, sic_fields):
+        """One member's {config name: (X, Y, Tfull) SIC field}, or a list of them -> float64 [members * n_configs][X * Y]
+        [Tfull]; raises ValueError unless the member count and shapes are the sweep's."""
+        member_fields = _members(sic_fields, 1)
+        if len(member_fields) != self.members:
+            raise ValueError(f"{len(member_fields)} members given, the sweep was built for {self.members}")
+        for mf in member_fields:
+            for c in self.cfgs:
+                if np.shape(mf[c.name]) != (self.X, self.Y, self.Tfull):
+                    raise ValueError(f"{c.name}: SIC field of shape {np.shape(mf[c.name])}, expected "
+                                     f"{(self.X, self.Y, self.Tfull)}")
+        return np.stack([np.ascontiguousarray(mf[c.name], dtype=np.float64).reshape(self.X * self.Y, self.Tfull)
+                         for mf in member_fields for c in self.cfgs])
+
+    def _stack_sst(self, sst_field):
+        """One (Xs, Ys, Tfull) SST field shared by every member, or one per member -> float64 [members][Xs * Ys][Tfull];
+        raises ValueError unless the field count and shapes are the sweep's."""
+        sst_members = _members(sst_field, self.members)
+        if len(sst_members) != self.members:
+            raise ValueError(f"{len(sst_members)} SST fields given, the sweep was built for {self.members} members")
+        if any(np.shape(f) != (self.Xs, self.Ys, self.Tfull) for f in sst_members):
+            raise ValueError(f"SST fields must have the shape {(self.Xs, self.Ys, self.Tfull)}")
+        return np.stack([np.ascontiguousarray(f, dtype=np.float64).reshape(self.Xs * self.Ys, self.Tfull)
+                         for f in sst_members])
+
+    def _device_inputs(self):
+        """A device buffer for every pinned input."""
+        return {k: torch.empty_like(t, device="cuda") for k, t in self._pin.items()}
 
     def _host_inputs(self):
         p = self.plan
@@ -753,19 +783,11 @@ class RetrospectiveSweep:
         return int(sum(t.numel() * t.element_size() for t in self._pin.values()))
 
     def d2h_bytes(self):
-        if self.tune is None:
-            sel = 0
-        elif self.hyper_mode == "argmin":
-            sel = self.P * (GP_PROBLEM_DTYPE.itemsize + 4)                      # tuned problems + best
-        else:
-            sel = self.P * (GP_MARGINAL_DTYPE.itemsize + 8 * self.levels.size)  # stats + quantiles
-        return int(self.P * GP_RESULT_DTYPE.itemsize + sel)
+        return int(sum(t.numel() * t.element_size() for t in self._d2h))
 
     def upload(self):
         """Host -> device copy of every input (pinned, async on the current stream) into device buffers that keep their
         addresses, so the captured step (compute) can be replayed on fresh inputs."""
-        if getattr(self, "dev", None) is None:
-            self.dev = {k: torch.empty_like(t, device="cuda") for k, t in self._pin.items()}
         for k, t in self._pin.items():
             self.dev[k].copy_(t, non_blocking=True)
         self._h2d_done = torch.cuda.Event()
@@ -778,25 +800,8 @@ class RetrospectiveSweep:
         re-allocating them (the stored correlation matrices alone are ~29 GB for 8 north members).  Rewrites the pinned
         host buffers in place once every copy still reading them has finished.  `sst_field` None keeps the current SST
         inputs.  The node capacity stays the constructor's: a batch with more ocean cells raises in check_status()."""
-        member_fields = list(sic_fields) if isinstance(sic_fields, (list, tuple)) else [sic_fields]
-        if len(member_fields) != self.members:
-            raise ValueError(f"{len(member_fields)} members given, the sweep was built for {self.members}")
-        for mf in member_fields:
-            for c in self.cfgs:
-                if np.shape(mf[c.name]) != (self.X, self.Y, self.Tfull):
-                    raise ValueError(f"{c.name}: SIC field of shape {np.shape(mf[c.name])}, expected "
-                                     f"{(self.X, self.Y, self.Tfull)}")
-        sic = np.stack([np.ascontiguousarray(mf[c.name], dtype=np.float64).reshape(self.X * self.Y, self.Tfull)
-                        for mf in member_fields for c in self.cfgs])
-        sst = None
-        if self.use_sst and sst_field is not None:
-            sst_members = list(sst_field) if isinstance(sst_field, (list, tuple)) else [sst_field] * self.members
-            if len(sst_members) != self.members:
-                raise ValueError(f"{len(sst_members)} SST fields given, the sweep was built for {self.members} members")
-            if any(np.shape(f) != (self.Xs, self.Ys, self.Tfull) for f in sst_members):
-                raise ValueError(f"SST fields must have the shape {(self.Xs, self.Ys, self.Tfull)}")
-            sst = np.stack([np.ascontiguousarray(f, dtype=np.float64).reshape(self.Xs * self.Ys, self.Tfull)
-                            for f in sst_members])
+        sic = self._stack_sic(sic_fields)
+        sst = self._stack_sst(sst_field) if self.use_sst and sst_field is not None else None
         if self._h2d_done is not None:
             self._h2d_done.synchronize()
         self.sic_host = sic
@@ -1010,18 +1015,34 @@ class RetrospectiveSweep:
                 per_gp * (pr[1] > split)
         return int(n)
 
+    def _read_back(self, slot):
+        """Enqueue (current stream) the copies of the step's outputs self._d2h into pinned set `slot` -> the set."""
+        bufs = self._pinned[slot]
+        if bufs is None:
+            bufs = self._pinned[slot] = [torch.empty(t.shape, dtype=t.dtype, pin_memory=True) for t in self._d2h]
+        for b, t in zip(bufs, self._d2h):
+            b.copy_(t, non_blocking=True)
+        return bufs
+
+    def _decode(self, bufs):
+        """Host copies of self._d2h -> self.raw (a copy: the pinned buffers are reused), self.selection (tuned sweep),
+        self.marginal (marginal sweep)."""
+        host = [b.numpy() for b in bufs]
+        self.raw = host[0].view(GP_RESULT_DTYPE).copy()
+        if self.hyper_mode == "argmin":
+            self.selection = selection_records(host[1].view(GP_PROBLEM_DTYPE), host[2])
+        elif self.hyper_mode == "marginal":
+            self.marginal = marginal_records(host[1], host[2])
+
     def download(self):
         """Device -> host read of the GP results (synchronises).  Raises if any network build or GP problem ran out of
         the capacity this sweep was sized for (a silent NaN forecast would look like a reference failure).  Tuned
         sweep: also reads the selected (l, sigma_n~) and grid indices into self.selection; marginal sweep: the grid
         posterior's stats and the quantiles into self.marginal."""
-        self.raw = self.gp.results()[:self.P]
+        bufs = self._read_back(2)
+        torch.cuda.current_stream().synchronize()
+        self._decode(bufs)
         self.check_status(self.raw)
-        if self.hyper_mode == "argmin":
-            self.selection = selection_records(self.tuned_problems(), self.best_index())
-        elif self.hyper_mode == "marginal":
-            self.marginal = marginal_records(self._mstats.cpu().numpy(),
-                                             self._quant.cpu().numpy()[:self.P * self.levels.size])
         return self.raw
 
     def run(self):
@@ -1036,27 +1057,13 @@ class RetrospectiveSweep:
         device, so host work (launch enqueue, assemble) is off the device's critical path, and step i+1's inputs are
         copied from the pinned buffers into a second set of device buffers on a copy stream while step i computes.
         Yields the same dict as run() per step; `self.raw` holds the records of the step just yielded."""
-        if getattr(self, "_pin_out", None) is None:
-            self._pin_out = [torch.empty(self.gp.out.numel(), dtype=torch.uint8).pin_memory() for _ in range(2)]
-        if self.hyper_mode == "argmin" and getattr(self, "_pin_sel", None) is None:
-            self._pin_sel = [(torch.empty(self._tuned.numel(), dtype=torch.uint8).pin_memory(),
-                              torch.empty(self.P, dtype=torch.int32).pin_memory()) for _ in range(2)]
-        if self.hyper_mode == "marginal" and getattr(self, "_pin_marg", None) is None:
-            self._pin_marg = [(torch.empty(self._mstats.numel(), dtype=torch.uint8).pin_memory(),
-                               torch.empty(self._quant.numel(), dtype=torch.float64).pin_memory()) for _ in range(2)]
         pending = None
 
-        def finish(ev, buf, k):
+        def finish(ev, k):
             ev.synchronize()
-            self.raw = buf.numpy().view(GP_RESULT_DTYPE)[:self.P].copy()    # the buffer is reused two steps later
+            self._decode(self._pinned[k])
             if (self.raw["info"] == -2).any():
                 self.check_status(self.raw)
-            if self.hyper_mode == "argmin":
-                tp, bp = self._pin_sel[k]
-                self.selection = selection_records(tp.numpy().view(GP_PROBLEM_DTYPE), bp.numpy())
-            elif self.hyper_mode == "marginal":
-                sp, qp = self._pin_marg[k]
-                self.marginal = marginal_records(sp.numpy(), qp.numpy()[:self.P * self.levels.size])
             return self.plan.assemble(self.raw, selection=self.selection, marginal=self.marginal)
 
         # inputs are double-buffered on the device: step i+1's host -> device copy runs on a copy stream while step i
@@ -1064,10 +1071,8 @@ class RetrospectiveSweep:
         n = int(n)
         overlap = not self.use_graph
         if overlap:
-            if getattr(self, "dev", None) is None:
-                self.dev = {k: torch.empty_like(t, device="cuda") for k, t in self._pin.items()}
-            if getattr(self, "_dev2", None) is None:
-                self._dev2 = {k: torch.empty_like(t, device="cuda") for k, t in self._pin.items()}
+            if self._dev2 is None:
+                self._dev2 = self._device_inputs()
                 self._copy_stream = torch.cuda.Stream()
             devs = [self.dev, self._dev2]
             main = torch.cuda.current_stream()
@@ -1102,21 +1107,12 @@ class RetrospectiveSweep:
             else:
                 self.upload()
                 self.compute()
-            buf = self._pin_out[i & 1]
-            buf.copy_(self.gp.out, non_blocking=True)
-            if self.hyper_mode == "argmin":
-                tp, bp = self._pin_sel[i & 1]
-                tp.copy_(self._tuned, non_blocking=True)
-                bp.copy_(self._best, non_blocking=True)
-            elif self.hyper_mode == "marginal":
-                sp, qp = self._pin_marg[i & 1]
-                sp.copy_(self._mstats, non_blocking=True)
-                qp.copy_(self._quant, non_blocking=True)
+            self._read_back(i & 1)
             ev = torch.cuda.Event()
             ev.record()
             if pending is not None:
                 yield finish(*pending)
-            pending = (ev, buf, i & 1)
+            pending = (ev, i & 1)
         if pending is not None:
             yield finish(*pending)
         self.check_status()                    # every step ran the same inputs: one check of the job statuses suffices

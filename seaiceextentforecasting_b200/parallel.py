@@ -19,6 +19,10 @@ import torch.distributed as dist
 TILE_ROWS = 128     # csrc/corr.cu TILE
 
 
+def _multi_rank(group=None):
+    return dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1
+
+
 def shard_tile_rows(n_nodes, rank, count):
     """Tile rows (128 nodes each) of the upper triangle computed by `rank` of `count` (csrc/corr.cu shard_rows)."""
     nb = (int(n_nodes) + TILE_ROWS - 1) // TILE_ROWS
@@ -30,7 +34,7 @@ def tau_from_shards(tau_sum, tau_cnt, group=None):
     (ComplexNetworks.py:45-47: mean of the significant non-negative correlations over both triangles)."""
     s = tau_sum.clone()
     c = tau_cnt.clone()
-    if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
+    if _multi_rank(group):
         dist.all_reduce(s, op=dist.ReduceOp.SUM, group=group)
         dist.all_reduce(c, op=dist.ReduceOp.SUM, group=group)
     return s / c.to(torch.float64)
@@ -48,7 +52,7 @@ def network_state(eng):
 def broadcast_networks(state, src=0, group=None):
     """Broadcast every tensor of `state` (network_state of an engine, or CPU tensors under gloo) from rank `src`
     in place.  Used after a network whose correlation pass was row-sharded has been grown on one rank."""
-    if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
+    if _multi_rank(group):
         for k in NETWORK_TENSORS:
             dist.broadcast(state[k], src=src, group=group)
     return state
@@ -58,7 +62,7 @@ def all_gather_networks(state, n_jobs_total, group=None):
     """Rank r built the networks (jobs) r, r + world, r + 2 world, ... of a sweep in a LOCAL batch (`state`: its
     network_state, job-major).  Returns the same tensors for ALL `n_jobs_total` jobs in global job order on every rank:
     one all-gather per tensor of labels / area tables / node series (a few hundred KB per 25 km network)."""
-    if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1:
+    if not _multi_rank(group):
         return {k: state[k][:n_jobs_total] for k in NETWORK_TENSORS}
     world = dist.get_world_size(group)
     per = (n_jobs_total + world - 1) // world
@@ -98,6 +102,29 @@ def build_networks_sharded(eng, fields, job_field, job_T, r_crit, scale, do_detr
     return eng.tau
 
 
+def _gather_rows(rows, group, device, rows_dev=None):
+    """Tensor all-gather of an array whose length (first axis) differs between ranks: the lengths are gathered first
+    and the payloads padded to the longest.  Returns the concatenation in rank order.  `rows_dev`: the payload as a
+    uint8 device tensor instead of the bytes of `rows` (which then only gives the length, dtype and row shape)."""
+    if device is None:
+        device = "cuda" if dist.get_backend(group) == "nccl" else "cpu"
+    rows = np.ascontiguousarray(rows)
+    rsz = rows.dtype.itemsize * int(np.prod(rows.shape[1:]))            # bytes per row
+    n = torch.tensor([len(rows)], dtype=torch.int64, device=device)
+    counts = [torch.zeros_like(n) for _ in range(dist.get_world_size(group))]
+    dist.all_gather(counts, n, group=group)
+    counts = [int(c.item()) for c in counts]
+    pay = torch.zeros(max(max(counts), 1) * rsz, dtype=torch.uint8, device=device)
+    if rows_dev is not None:
+        pay[:len(rows) * rsz] = rows_dev[:len(rows) * rsz].to(device)
+    else:
+        pay[:len(rows) * rsz] = torch.from_numpy(rows.view(np.uint8).reshape(-1).copy()).to(device)
+    pays = [torch.empty_like(pay) for _ in counts]
+    dist.all_gather(pays, pay, group=group)
+    return np.concatenate([p.cpu().numpy()[:c * rsz].view(rows.dtype).reshape((c,) + rows.shape[1:])
+                           for p, c in zip(pays, counts)])
+
+
 def gather_records(plan, raw, group=None, device=None, raw_dev=None):
     """Tensor all-gather of every rank's GP records (80 B each) and their (config, region, year, member) keys: ranks
     own different numbers of problems, so the counts are gathered first and the payloads padded to the largest.
@@ -107,35 +134,15 @@ def gather_records(plan, raw, group=None, device=None, raw_dev=None):
     from .forecast import GP_RESULT_DTYPE
     if raw is None:
         raw = np.zeros(plan.P, dtype=GP_RESULT_DTYPE) if raw_dev is not None else np.zeros(0, dtype=GP_RESULT_DTYPE)
-        if raw_dev is not None and not (dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1):
+        if raw_dev is not None and not _multi_rank(group):
             raw = raw_dev.cpu().numpy().view(GP_RESULT_DTYPE)[:plan.P]
     raw = np.ascontiguousarray(raw)
     meta = np.asarray(plan.prob_meta, dtype=np.int32).reshape(-1, 3)
     keys = np.concatenate([meta, np.asarray(plan.prob_member, dtype=np.int32).reshape(-1, 1)], axis=1)
-    if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1:
+    if not _multi_rank(group):
         return raw, keys[:, :3], keys[:, 3]
-    world = dist.get_world_size(group)
-    if device is None:
-        device = "cuda" if dist.get_backend(group) == "nccl" else "cpu"
-    isz = raw.dtype.itemsize
-    n = torch.tensor([len(raw)], dtype=torch.int64, device=device)
-    counts = [torch.zeros_like(n) for _ in range(world)]
-    dist.all_gather(counts, n, group=group)
-    counts = [int(c.item()) for c in counts]
-    cap = max(max(counts), 1)
-    pay = torch.zeros(cap * isz, dtype=torch.uint8, device=device)
-    if raw_dev is not None:
-        pay[:len(raw) * isz] = raw_dev[:len(raw) * isz].to(device)
-    else:
-        pay[:len(raw) * isz] = torch.from_numpy(raw.view(np.uint8).reshape(-1).copy()).to(device)
-    key = torch.zeros((cap, 4), dtype=torch.int32, device=device)
-    key[:len(raw)] = torch.from_numpy(np.ascontiguousarray(keys)).to(device)
-    pays = [torch.empty_like(pay) for _ in range(world)]
-    keyl = [torch.empty_like(key) for _ in range(world)]
-    dist.all_gather(pays, pay, group=group)
-    dist.all_gather(keyl, key, group=group)
-    raw_all = np.concatenate([p.cpu().numpy()[:c * isz].view(raw.dtype) for p, c in zip(pays, counts)])
-    key_all = np.concatenate([k.cpu().numpy()[:c] for k, c in zip(keyl, counts)])
+    raw_all = _gather_rows(raw, group, device, raw_dev)
+    key_all = _gather_rows(keys, group, device)
     return raw_all, key_all[:, :3], key_all[:, 3]
 
 
@@ -145,21 +152,7 @@ def gather_selection(selection, group=None, device=None):
     rank assembles the same tuned dict.  Any structured per-problem array gathers the same way (the marginal records
     of a marginalised sweep)."""
     sel = np.ascontiguousarray(selection)
-    if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1:
-        return sel
-    world = dist.get_world_size(group)
-    if device is None:
-        device = "cuda" if dist.get_backend(group) == "nccl" else "cpu"
-    isz = sel.dtype.itemsize
-    n = torch.tensor([len(sel)], dtype=torch.int64, device=device)
-    counts = [torch.zeros_like(n) for _ in range(world)]
-    dist.all_gather(counts, n, group=group)
-    counts = [int(c.item()) for c in counts]
-    pay = torch.zeros(max(max(counts), 1) * isz, dtype=torch.uint8, device=device)
-    pay[:len(sel) * isz] = torch.from_numpy(sel.view(np.uint8).reshape(-1).copy()).to(device)
-    pays = [torch.empty_like(pay) for _ in range(world)]
-    dist.all_gather(pays, pay, group=group)
-    return np.concatenate([p.cpu().numpy()[:c * isz].view(sel.dtype) for p, c in zip(pays, counts)])
+    return _gather_rows(sel, group, device) if _multi_rank(group) else sel
 
 
 def gather_results(plan, raw, group=None, device=None, selection=None, marginal=None):

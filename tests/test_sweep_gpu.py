@@ -233,6 +233,7 @@ def test_run_many_equals_run(lib_built):
         for cfg in ref:
             for k, v in ref[cfg].items():
                 assert np.array_equal(np.asarray(out[cfg][k]), np.asarray(v), equal_nan=True), (cfg, k)
+    assert sw.d2h_bytes() == sw.P * 80
 
 
 def test_full_size_north_sweep_invariants(lib_built):

@@ -186,6 +186,7 @@ def test_tuned_records_do_not_depend_on_the_schedule(tuned_small):
         for c in outs[0]:
             for k, v in outs[0][c].items():
                 assert np.array_equal(o[c][k], v, equal_nan=True), (c, k)
+    assert sw.d2h_bytes() == sw.P * (80 + 56 + 4)
 
 
 def test_load_inputs_streams_a_new_member(lib_built):
