@@ -168,10 +168,8 @@ class NetworkBatch:
                                        _ptr(self.n_nodes[j0:]), n, self.X, self.Y, self.ldn, int(self.latlon),
                                        _ptr(self.stencil[j0:]), _stream())
         _lib.check(rc, "sie_corr_stencil")
-        scratch = self._area_scratch.get((j0, j1))            # ranges may run concurrently: one scratch each
-        if scratch is None:
-            nbytes = int(self.lib.sie_area_level_scratch_bytes(n, self.C))
-            scratch = self._area_scratch[(j0, j1)] = torch.empty((nbytes + 7) // 8, dtype=torch.float64, device="cuda")
+        self.prepare([(j0, j1)])
+        scratch = self._area_scratch[(j0, j1)]                # ranges may run concurrently: one scratch each
         rc = self.lib.sie_area_level(R, _ptr(self.z[j0:]), _ptr(self.job_T[j0:]), self.Tp,
                                      _ptr(self.stencil[j0:]), _ptr(self.node_cell[j0:]),
                                      _ptr(self.cell_node[j0:]), _ptr(self.n_nodes[j0:]), _ptr(self.tau[j0:]),
@@ -183,12 +181,25 @@ class NetworkBatch:
         _lib.check(rc, "sie_area_level")
         self.launches += 2
 
-    def prepare(self, ranges=None):
-        """Allocate the per-range scratch up front (compute() may be captured into a CUDA graph: no allocation there)."""
-        for (j0, j1) in (ranges or [(0, self.B)]):
-            if (j0, j1) not in self._area_scratch and j1 > j0:
-                nbytes = int(self.lib.sie_area_level_scratch_bytes(j1 - j0, self.C))
-                self._area_scratch[(j0, j1)] = torch.empty((nbytes + 7) // 8, dtype=torch.float64, device="cuda")
+    def prepare(self, *schedules):
+        """Allocate the domain-growth scratch of job ranges (j0, j1) that have none yet; area_level() does so on a
+        range's first use, a caller that captures its stages into a CUDA graph calls this up front.  Every schedule is
+        a list of ranges that may run concurrently, so they get disjoint scratch; different schedules run one at a time
+        (stream order), so they share one allocation."""
+        layout, end = {}, 0                     # range -> (offset, float64 count) in the shared allocation
+        for ranges in schedules:
+            new = [r for r in map(tuple, ranges) if r[1] > r[0] and r not in self._area_scratch]
+            off = end if any(r in layout for r in new) else 0      # a range placed by an earlier schedule stays put
+            for r in new:
+                if r not in layout:
+                    n = (int(self.lib.sie_area_level_scratch_bytes(r[1] - r[0], self.C)) + 7) // 8
+                    layout[r] = (off, n)
+                    off += (n + 63) // 64 * 64                      # 512-byte aligned slices
+            end = max(end, off)
+        if layout:
+            buf = torch.empty(end, dtype=torch.float64, device="cuda")
+            for r, (off, n) in layout.items():
+                self._area_scratch[r] = buf[off:off + n]
 
     def intra_links(self, scale, jr=None):
         """K6.  scale: device float64 [C] (already square-rooted weights)."""

@@ -8,9 +8,8 @@ forecast :208-288; MLII :235-257; read_SIE de-trending June1st_retro.py:58-69; s
 """
 from __future__ import annotations
 
+import collections
 import ctypes as C
-
-import os
 import weakref
 
 import numpy as np
@@ -128,10 +127,13 @@ class GpBatch:
                                       _stream())
         _lib.check(rc, "sie_gp_forecast")
 
-    def run_grid(self, prob_dev, sig_grid_dev, n_sig, y_dev, sic, sst, out):
+    def run_grid(self, prob_dev, sig_grid_dev, n_sig, y_dev, sic, sst, out, n=None):
         """Hyper-parameter grid: problem p fixes l = prob[p].ell; every sig_grid[k] is evaluated from the same
-        expm / X Sigma X^T (sie_gp_hyper_grid).  `out`: uint8 device buffer of P * n_sig result records."""
-        rc = self.lib.sie_gp_hyper_grid(_ptr(prob_dev), self.P, _ptr(sig_grid_dev), int(n_sig), _ptr(y_dev),
+        expm / X Sigma X^T (sie_gp_hyper_grid).  `n`: run the first n <= P problems of prob_dev (default: P).  `out`:
+        uint8 device buffer of n * n_sig result records."""
+        n = self.P if n is None else int(n)
+        assert 0 < n <= self.P
+        rc = self.lib.sie_gp_hyper_grid(_ptr(prob_dev), n, _ptr(sig_grid_dev), int(n_sig), _ptr(y_dev),
                                         *_series_args(sic, sst), self.max_pred, _ptr(out), _ptr(self.scratch),
                                         self.scratch_bytes, _stream())
         _lib.check(rc, "sie_gp_hyper_grid")
@@ -594,6 +596,13 @@ def _members(x, n):
     return list(x) if isinstance(x, (list, tuple)) else [x] * n
 
 
+# One GP launch of a sweep step: its wave, its problems p0..p1-1, whether it reads SST networks (it then also waits for
+# them and runs on its wave's SST stream) and the GpBatch whose scratch it runs on
+_Launch = collections.namedtuple("_Launch", "wave p0 p1 sst gp")
+# A step's schedule: its waves (job range, SST job range, problem range) and its GP launches in enqueue order
+_Plan = collections.namedtuple("_Plan", "waves launches")
+
+
 class RetrospectiveSweep:
     """years fmin..fmax x the given init-month configs x 3 regions, in one device-resident batch.
 
@@ -657,15 +666,29 @@ class RetrospectiveSweep:
                                     max_areas=max_areas, keep_R=keep_R)
         self.P = plan.P
         self.n_forecasts = plan.P
-        self.gp = GpBatch(max(1, self.P), max_pred=max_pred)
-        self._side = None
+        self._grids = {}                       # (ells, sigs) -> _GridBuffers (hyper_grid() and the tuned step)
+        self.tune = None
+        self.hyper_mode = hyper_mode if hyper_grid is not None else None
+        self.levels = levels
+        self.selection = None                  # tuned mode: SELECTION_DTYPE [P] of the step last read back
+        self.marginal = None                   # marginal mode: marginal_dtype(n_q) [P] of the step last read back
+        if hyper_grid is not None:
+            ells, sigs = (np.ascontiguousarray(a, dtype=np.float64).reshape(-1) for a in hyper_grid)
+            if ells.size < 1 or sigs.size < 1 or self.P < 1:
+                raise ValueError("hyper_grid needs at least one l and one sigma_n~ value and a sweep with problems")
+            self.tune = self._grid_buffers(ells, sigs)
+            if hyper_mode == "argmin":
+                self._tuned = torch.empty(self.P * GP_PROBLEM_DTYPE.itemsize, dtype=torch.uint8, device="cuda")
+                self._best = torch.empty(self.P, dtype=torch.int32, device="cuda")
+            else:
+                self._q_dev = h2d(levels) if levels.size else None
+                self._mstats = torch.empty(self.P * GP_MARGINAL_DTYPE.itemsize, dtype=torch.uint8, device="cuda")
+                self._quant = torch.empty(max(1, self.P * levels.size), dtype=torch.float64, device="cuda")
         # Waves.  Jobs and GP problems are ordered by descending year, so splitting the window lengths at `wave_T` edges
         # gives contiguous job / problem ranges: wave 0 = the longest windows (slowest domain growth, small GP problems),
         # the last wave = the shortest windows (networks finish early; their many small areas give the expensive
         # 100-160-predictor GP problems).  Every wave runs its chain on its own stream and its GP starts as soon as ITS
         # networks are done, overlapping the domain growth of the longer-window waves.
-        if os.environ.get("SIE_WAVE_T"):          # tuning override, e.g. SIE_WAVE_T=16 or 12,24
-            wave_T = tuple(int(x) for x in os.environ["SIE_WAVE_T"].split(","))
         edges = sorted({int(e) for e in (wave_T if isinstance(wave_T, (tuple, list)) else (wave_T,))}, reverse=True)
         self.wave_T = tuple(edges)
         T = plan.job_T
@@ -693,45 +716,45 @@ class RetrospectiveSweep:
             for (jr, sr, pr) in self.waves:
                 ok = ok and bool((plan.prob["job_sic"][pr[0]:pr[1]] >= jr[0]).all())
         self.multi_wave = bool(ok and len(self.waves) > 1)
-        self.gp_wave = [GpBatch(max(1, pr[1] - pr[0]), max_pred=max_pred) for (_, _, pr) in self.waves[1:]] \
-            if self.multi_wave else []
-        # Within a wave the problems that read no SST network come first: they only wait for the wave's SIC networks,
-        # the SST-reading ones (June) also for its SST networks, which finish later - two GP launches per wave instead
-        # of one that waits for everything.  Records are self-contained (y_off), so this is a permutation of
-        # plan.prob / plan.prob_meta; assemble() looks results up through prob_meta.
-        self.psplit = [pr[1] for (_, _, pr) in self.waves]
-        self.gp_sst = []
-        if self.multi_wave and self.use_sst and not os.environ.get("SIE_NO_GP_SPLIT"):
-            self.psplit = plan.partition_sst([pr for (_, _, pr) in self.waves])
-            self.gp_sst = [GpBatch(max(1, pr[1] - self.psplit[w]), max_pred=max_pred) for w, (_, _, pr) in enumerate(self.waves)]
-        self._streams = None
+        # The launch plan of a step, built here so that compute() only walks it and allocates nothing: the waves (job,
+        # SST job and problem ranges) and the GP launches in enqueue order.  Within a wave of a multi-wave step the
+        # problems that read no SST network come first: they only wait for the wave's SIC networks, the SST-reading ones
+        # (June) also for its SST networks, which finish later - two GP launches per wave instead of one that waits for
+        # everything (13.0 -> 12.5 ms, DESIGN.md section 6).  Records are self-contained (y_off), so this is a
+        # permutation of plan.prob / plan.prob_meta; assemble() looks results up through prob_meta.
+        self.gp_sst = self.multi_wave and self.use_sst          # the SST split is on
+        ranges = [pr for (_, _, pr) in self.waves]
+        splits = plan.partition_sst(ranges) if self.gp_sst else [p1 for (_, p1) in ranges]
+        # a grid-mode launch runs (p1 - p0) * n_ell grid problems on its batch, whose scratch also serves its forecast
+        n_ell = 1 if self.tune is None else len(self.tune.ells)
+        # the launch from problem 0 runs on self.gp, sized for all P so that the one-wave plan reuses it; self.gp.out
+        # receives every launch's records
+        self.gp = GpBatch(max(1, self.P) * n_ell, max_pred=max_pred)
+        self._one_wave = _Plan([((0, self.sic.B), (0, self.sst.B if self.use_sst else 0), (0, self.P))],
+                               [_Launch(0, 0, self.P, self.use_sst, self.gp)] if self.P else [])
+        self._plan = self._one_wave
+        if self.multi_wave:
+            launches = []
+            for w in range(len(ranges) - 1, -1, -1):
+                p0, p1 = ranges[w]
+                for lo, hi, sst in ((p0, splits[w], False), (splits[w], p1, True)):
+                    if hi > lo:
+                        gp = self.gp if lo == 0 else GpBatch((hi - lo) * n_ell, max_pred=max_pred)
+                        launches.append(_Launch(w, lo, hi, sst, gp))
+            self._plan = _Plan(self.waves, launches)
+        self._streams = [(torch.cuda.Stream(priority=-1), torch.cuda.Stream(priority=-1)) for _ in self._plan.waves]
+        plans = (self._plan, self._one_wave)   # steps run one at a time: the plans share their domain-growth scratch
+        self.sic.prepare(*[[jr for (jr, _, _) in p.waves] for p in plans])
+        if self.use_sst:
+            self.sst.prepare(*[[sr for (_, sr, _) in p.waves] for p in plans])
         self._graph = None
-        self.use_graph = bool(os.environ.get("SIE_GRAPH"))      # opt-in: see compute()
+        self.use_graph = False                 # opt-in: see compute()
         # pinned staging buffers so every step pays a real host->device copy
         self._pin = {name: torch.from_numpy(np.ascontiguousarray(arr)).pin_memory()
                      for name, arr in self._host_inputs().items()}
         self.dev = self._device_inputs()
         self._dev2, self._copy_stream = None, None     # run_many's second input set and its copy stream
         self._h2d_done = None                  # event after the last enqueued copy out of self._pin (load_inputs)
-        self._grids = {}                       # (ells, sigs) -> _GridBuffers (hyper_grid() and the tuned step)
-        self.tune = None
-        self.hyper_mode = hyper_mode if hyper_grid is not None else None
-        self.levels = levels
-        self.selection = None                  # tuned mode: SELECTION_DTYPE [P] of the step last read back
-        self.marginal = None                   # marginal mode: marginal_dtype(n_q) [P] of the step last read back
-        if hyper_grid is not None:
-            ells, sigs = (np.ascontiguousarray(a, dtype=np.float64).reshape(-1) for a in hyper_grid)
-            if ells.size < 1 or sigs.size < 1 or self.P < 1:
-                raise ValueError("hyper_grid needs at least one l and one sigma_n~ value and a sweep with problems")
-            self.tune = self._grid_buffers(ells, sigs)
-            if hyper_mode == "argmin":
-                self._tuned = torch.empty(self.P * GP_PROBLEM_DTYPE.itemsize, dtype=torch.uint8, device="cuda")
-                self._best = torch.empty(self.P, dtype=torch.int32, device="cuda")
-            else:
-                self._q_dev = h2d(levels) if levels.size else None
-                self._mstats = torch.empty(self.P * GP_MARGINAL_DTYPE.itemsize, dtype=torch.uint8, device="cuda")
-                self._quant = torch.empty(max(1, self.P * levels.size), dtype=torch.float64, device="cuda")
-            self._gp_tuned = {}                # GP launch range -> GpBatch of its grid (its scratch also serves the forecast)
         # what a step reads back, each sliced to the bytes read (decoded by _decode); pinned host copies per slot:
         # 0 / 1 for run_many's two steps in flight, 2 for download()
         self._d2h = [self.gp.out[:self.P * GP_RESULT_DTYPE.itemsize]]
@@ -812,17 +835,20 @@ class RetrospectiveSweep:
 
     def compute(self, marks=None, waves=None):
         """Enqueue the whole hot path on the current stream (no host sync).  `marks`: optional list that receives
-        (stage name, torch.cuda.Event) pairs recorded after each stage, for per-kernel timing.  `waves`: 0 = every
-        stage alone on one stream (clean per-stage timing), 1 = one batch per grid with the SST chain on a side stream,
-        2 = short/long-window waves on separate streams (default when possible).
-        With `use_graph` (SIE_GRAPH=1) the default call (no marks, default waves) is captured once into a CUDA graph -
+        (stage name, torch.cuda.Event) pairs recorded after each stage, for per-kernel timing.  `waves`: None = the
+        launch plan's waves (short/long-window waves on separate streams when the sweep is multi-wave), 1 = one wave:
+        one SIC chain and one SST chain on two streams and one GP launch that waits for both, 0 = that one wave with
+        every stage on the current stream (clean per-stage timing).
+        With `use_graph` the default call (no marks, default waves) is captured once into a CUDA graph -
         ~55 kernels on up to five streams with their cross-stream dependencies - and replayed afterwards: one launch
         per step instead of ~150 ctypes / stream calls.  Measured on B200 (same box, N = 1 and 2): the replayed step is
         ~5 % SLOWER back to back (13.8 vs 12.9 ms; the graph's branch scheduling loses the issue order the eager
         streams impose) and ~1 % faster end to end, so eager stays the default."""
+        if waves not in (None, 0, 1):
+            raise ValueError(f"waves must be None, 0 or 1, got {waves!r}")
         if marks is None and waves is None and self.use_graph:
             if self._graph is None:
-                self._compute(None, None)               # eager once: creates the streams, sets the kernel attributes
+                self._compute(None, None)               # eager once: sets the kernel attributes
                 torch.cuda.synchronize()
                 g = torch.cuda.CUDAGraph()
                 with torch.cuda.graph(g):
@@ -834,7 +860,11 @@ class RetrospectiveSweep:
 
     def _compute(self, marks, waves):
         d = self.dev
-        two = self.multi_wave if waves is None else (waves != 1 and self.multi_wave)
+        plan_waves, launches = self._plan if waves is None else self._one_wave
+        nw = len(plan_waves)
+        sfx = [""] if nw == 1 else [str(w) for w in range(nw)]        # stage tags: sic / sst / gp, or sic0, gps1, ...
+        main = torch.cuda.current_stream()
+        streams = [(main, main)] if waves == 0 else self._streams[:nw]
 
         def mark(name):
             if marks is not None:
@@ -842,7 +872,7 @@ class RetrospectiveSweep:
                 ev.record()
                 marks.append((name, ev))
 
-        def chain(tag, eng, fields, job_field, job_T, rcrit, scale, jr=None):
+        def chain(tag, eng, fields, job_field, job_T, rcrit, scale, jr):
             mark(tag + ".start")
             eng.detrend_zscore(fields, job_field, job_T, do_detrend=True, jr=jr)
             mark(tag + ".detrend_zscore")
@@ -853,38 +883,9 @@ class RetrospectiveSweep:
             eng.intra_links(scale, jr=jr)
             mark(tag + ".intra_links")
 
-        main = torch.cuda.current_stream()
         if self.tune is not None:               # before any side stream forks from `main`
             expand_problems(d["prob"], self.tune.ell_dev, self.tune.prob)
-        if waves == 0:
-            # fully serial on the current stream (per-stage timing: no other kernel shares the GPU with the timed stage)
-            if self.sst is not None:
-                chain("sst", self.sst, d["sst"], d["sst_field_idx"], d["sst_T"], d["sst_rcrit"], d["lat"])
-            chain("sic", self.sic, d["sic"], d["job_field"], d["job_T"], d["rcrit"], d["psar"])
-            mark("gp.start")
-            self._gp_run(self.gp, None, mark, "gp")
-            mark("gp")
-            return
-        if not two:
-            if self.sst is not None:
-                # the SST networks are independent of the SIC ones: run their chain on a side stream so the two
-                # latency-bound domain-growth kernels share the SMs instead of running back to back
-                if self._side is None:
-                    self._side = torch.cuda.Stream()
-                self._side.wait_stream(main)
-                with torch.cuda.stream(self._side):
-                    chain("sst", self.sst, d["sst"], d["sst_field_idx"], d["sst_T"], d["sst_rcrit"], d["lat"])
-            chain("sic", self.sic, d["sic"], d["job_field"], d["job_T"], d["rcrit"], d["psar"])
-            if self.sst is not None:
-                main.wait_stream(self._side)
-            mark("gp.start")
-            self._gp_run(self.gp, None, mark, "gp")
-            mark("gp")
-            return
-        nw = len(self.waves)
-        if self._streams is None:
-            self._streams = [(torch.cuda.Stream(priority=-1), torch.cuda.Stream(priority=-1)) for _ in range(nw)]
-        for (s1, s2) in self._streams:
+        for (s1, s2) in streams:
             s1.wait_stream(main)
             s2.wait_stream(main)
         sdone = [None] * nw                     # SST networks of wave w complete (None: the wave has none)
@@ -895,68 +896,52 @@ class RetrospectiveSweep:
         # 5-12 % slower in steady state: the long-window area CTAs must never wait for an SM)
         seq = [("s", w) for w in range(nw)] + [("t", w) for w in range(nw - 1, -1, -1)]
         for kind, w in seq:
-            jr, sr, pr = self.waves[w]
+            jr, sr, _ = plan_waves[w]
             if kind == "s":
-                with torch.cuda.stream(self._streams[w][0]):
+                with torch.cuda.stream(streams[w][0]):
                     if jr[1] > jr[0]:
-                        chain(f"sic{w}", self.sic, d["sic"], d["job_field"], d["job_T"], d["rcrit"], d["psar"], jr)
+                        chain("sic" + sfx[w], self.sic, d["sic"], d["job_field"], d["job_T"], d["rcrit"], d["psar"], jr)
                     ev = torch.cuda.Event()
                     ev.record()
                     done[w] = ev
-            elif self.sst is not None and sr[1] > sr[0]:
-                with torch.cuda.stream(self._streams[w][1]):
-                    chain(f"sst{w}", self.sst, d["sst"], d["sst_field_idx"], d["sst_T"], d["sst_rcrit"], d["lat"], sr)
+            elif sr[1] > sr[0]:
+                with torch.cuda.stream(streams[w][1]):
+                    chain("sst" + sfx[w], self.sst, d["sst"], d["sst_field_idx"], d["sst_T"], d["sst_rcrit"], d["lat"],
+                          sr)
                     ev = torch.cuda.Event()
                     ev.record()
                     sdone[w] = ev
         # GP of wave w: needs its own networks and those of the shorter-window waves (previous-year configurations);
-        # the problems that read SST networks are a second launch that also waits for those
-        gp_streams = self._streams
-        for w in range(nw - 1, -1, -1):
-            jr, sr, pr = self.waves[w]
-            split = self.psplit[w] if self.gp_sst else pr[1]
-            if split > pr[0]:
-                st = gp_streams[w][0]
-                with torch.cuda.stream(st):
-                    for v in range(w, nw):
-                        st.wait_event(done[v])
-                        if not self.gp_sst and sdone[v] is not None:
-                            st.wait_event(sdone[v])
-                    mark(f"gp{w}.start")
-                    gp = self.gp if w == 0 else self.gp_wave[w - 1]
-                    self._gp_run(gp, (pr[0], split), mark, f"gp{w}")
-                    mark(f"gp{w}")
-            if pr[1] > split:
-                st = gp_streams[w][1]
-                with torch.cuda.stream(st):
-                    for v in range(w, nw):
-                        st.wait_event(done[v])
-                        if sdone[v] is not None:
-                            st.wait_event(sdone[v])
-                    mark(f"gps{w}.start")
-                    self._gp_run(self.gp_sst[w], (split, pr[1]), mark, f"gps{w}")
-                    mark(f"gps{w}")
-        for (s1, s2) in self._streams:          # the step is complete on `main` once every wave has finished
+        # a launch that reads SST networks also waits for those
+        for launch in launches:
+            w = launch.wave
+            tag = ("gps" if launch.sst and nw > 1 else "gp") + sfx[w]
+            st = streams[w][launch.sst]
+            with torch.cuda.stream(st):
+                for v in range(w, nw):
+                    st.wait_event(done[v])
+                    if launch.sst and sdone[v] is not None:
+                        st.wait_event(sdone[v])
+                mark(tag + ".start")
+                self._gp_run(launch, mark, tag)
+                mark(tag)
+        for (s1, s2) in streams:                # the step is complete on `main` once every wave has finished
             main.wait_stream(s1)
             main.wait_stream(s2)
 
-    def _gp_run(self, gp, pr, mark, tag):
-        """One GP launch of the step on the current stream over problems pr = (p0, p1) (None: all), results into
-        self.gp.out.  Tuned sweep: sie_gp_hyper_grid over the range's expanded problems, sie_gp_grid_select, then
-        sie_gp_forecast of the selected problems -- three launches in stream order, no host sync.  Marginal sweep: the
-        grid, then sie_gp_grid_marginal straight into self.gp.out and the range's stats / quantiles."""
-        d = self.dev
+    def _gp_run(self, launch, mark, tag):
+        """One GP launch of the step on the current stream over its problems p0..p1-1, results into self.gp.out.
+        Tuned sweep: sie_gp_hyper_grid over the range's expanded problems, sie_gp_grid_select, then sie_gp_forecast of
+        the selected problems -- three launches in stream order on the launch's batch, no host sync.  Marginal sweep:
+        the grid, then sie_gp_grid_marginal straight into self.gp.out and the range's stats / quantiles."""
+        d, p0, p1, gp = self.dev, launch.p0, launch.p1, launch.gp
         if self.tune is None:
-            gp.run(d["prob"], d["y"], self.sic, self.sst, pr, out=self.gp.out)
+            gp.run(d["prob"], d["y"], self.sic, self.sst, (p0, p1), out=self.gp.out)
             return
-        p0, p1 = (0, self.P) if pr is None else (int(pr[0]), int(pr[1]))
         g, nl, ns = self.tune, len(self.tune.ells), len(self.tune.sigs)
         isz, osz = GP_PROBLEM_DTYPE.itemsize, GP_RESULT_DTYPE.itemsize
-        gx = self._gp_tuned.get((p0, p1))
-        if gx is None:                          # first (eager) step: allocated before any graph capture
-            gx = self._gp_tuned[(p0, p1)] = GpBatch((p1 - p0) * nl, max_pred=self.gp.max_pred)
         grid = g.out[p0 * nl * ns * osz:]
-        gx.run_grid(g.prob[p0 * nl * isz:], g.sig_dev, ns, d["y"], self.sic, self.sst, grid)
+        gp.run_grid(g.prob[p0 * nl * isz:], g.sig_dev, ns, d["y"], self.sic, self.sst, grid, n=(p1 - p0) * nl)
         mark(tag + ".grid")
         if self.hyper_mode == "marginal":
             nq = self.levels.size
@@ -964,7 +949,7 @@ class RetrospectiveSweep:
                           self._mstats[p0 * GP_MARGINAL_DTYPE.itemsize:], self._quant[p0 * nq:])
             return
         grid_select(grid, d["prob"][p0 * isz:], p1 - p0, g.ell_dev, g.sig_dev, self._tuned[p0 * isz:], self._best[p0:])
-        gx.run(self._tuned, d["y"], self.sic, self.sst, (p0, p1), out=self.gp.out)
+        gp.run(self._tuned, d["y"], self.sic, self.sst, (p0, p1), out=self.gp.out)
 
     def _grid_buffers(self, ells, sigs):
         key = (ells.tobytes(), sigs.tobytes())
@@ -1002,18 +987,11 @@ class RetrospectiveSweep:
         return g.out.cpu().numpy().view(GP_RESULT_DTYPE).reshape(self.P, nl, ns)
 
     def kernel_launches(self):
-        """Kernels of libsie_b200 enqueued by one compute(): 12 per network batch (K1: 3, K2: 4, K3-K5: 2, K6: 3), per
-        wave, + 2 per GP batch (tuned sweep: 5 -- grid 2, select 1, forecast 2; marginal sweep: 3 -- grid 2,
-        marginal 1)."""
+        """Kernels of libsie_b200 enqueued by one compute(): 12 per network chain (K1: 3, K2: 4, K3-K5: 2, K6: 3) + 2 per
+        GP launch (tuned sweep: 5 -- grid 2, select 1, forecast 2; marginal sweep: 3 -- grid 2, marginal 1)."""
         per_gp = 2 if self.tune is None else (5 if self.hyper_mode == "argmin" else 3)
-        if not self.multi_wave:
-            return 12 * (2 if self.use_sst else 1) + per_gp
-        n = 0
-        for w, (jr, sr, pr) in enumerate(self.waves):
-            split = self.psplit[w] if self.gp_sst else pr[1]
-            n += 12 * (jr[1] > jr[0]) + 12 * (self.use_sst and sr[1] > sr[0]) + per_gp * (split > pr[0]) + \
-                per_gp * (pr[1] > split)
-        return int(n)
+        chains = sum((jr[1] > jr[0]) + (sr[1] > sr[0]) for (jr, sr, _) in self._plan.waves)
+        return 12 * chains + per_gp * len(self._plan.launches)
 
     def _read_back(self, slot):
         """Enqueue (current stream) the copies of the step's outputs self._d2h into pinned set `slot` -> the set."""

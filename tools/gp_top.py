@@ -8,12 +8,11 @@ w = bench.make_workload(0)
 sw = RetrospectiveSweep(NORTH_INITS, w['sic'], w['sie'], bench.FMIN, bench.FMAX, w['psar'], w['sst'], w['lat'])
 sw.run(); sw.run()
 raw = sw.raw
-for wi, (jr, sr, pr) in enumerate(sw.waves):
-    for name, (a, b) in (("sic-only", (pr[0], sw.psplit[wi])), ("sst", (sw.psplit[wi], pr[1]))):
-        if b <= a: continue
-        idx = np.arange(a, b); c = raw["cycles_total"][idx] / 1e6
-        order = idx[np.argsort(-c)]
-        print(f"wave {wi} {name}: {b - a} problems, sum {c.sum():.1f} Mcyc, mean {c.mean():.3f}, max {c.max():.3f}")
-        for i in order[:8]:
-            print("   ", sw.plan.prob_meta[i], "n", sw.plan.prob[i]["n"], "Np", raw[i]["n_pred"], "m", raw[i]["expm_m"], "s", raw[i]["expm_s"],
-                  "total Mcyc", round(raw[i]["cycles_total"] / 1e6, 3), "expm", round(raw[i]["cycles_expm"] / 1e6, 3))
+for launch in sorted(sw._plan.launches, key=lambda l: l.p0):
+    wi, a, b, name = launch.wave, launch.p0, launch.p1, "sst" if launch.sst else "sic-only"
+    idx = np.arange(a, b); c = raw["cycles_total"][idx] / 1e6
+    order = idx[np.argsort(-c)]
+    print(f"wave {wi} {name}: {b - a} problems, sum {c.sum():.1f} Mcyc, mean {c.mean():.3f}, max {c.max():.3f}")
+    for i in order[:8]:
+        print("   ", sw.plan.prob_meta[i], "n", sw.plan.prob[i]["n"], "Np", raw[i]["n_pred"], "m", raw[i]["expm_m"], "s", raw[i]["expm_s"],
+              "total Mcyc", round(raw[i]["cycles_total"] / 1e6, 3), "expm", round(raw[i]["cycles_expm"] / 1e6, 3))
